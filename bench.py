@@ -3,6 +3,7 @@
 bench.py -- the contact-map hot path on N B200s (one process per GPU).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C1|C2|C3|C4]
+                    [--dump-outputs DIR]
 
 One "step" is one pass of the whole hot path over one batch of synthetic packed pair records:
 accumulate -> acceptance mask -> site normalisation -> Knight-Ruiz balancing -> compressed, scaled edge list.
@@ -48,6 +49,8 @@ DTYPE = 'u32 counts / f64 balancing'
 MIN_LEN, MIN_SIG = 1000, 5           # bin3C.py:27-34 runtime defaults
 CPU_SAMPLE_PAIRS = 50_000_000       # the whole of C2; a bounded prefix of the pair stream for larger configs
 REL_TOL = 1e-9                      # north_star: KR scale vector and edge weights
+DUMP_EDGES = 1_500_000              # --dump-outputs: u, v, w and their indices as float64 stay under 48 MB
+DUMP_SEED = 1234
 
 
 def parse_args():
@@ -70,7 +73,14 @@ def parse_args():
     ap.add_argument('--parity', default='sample', choices=['sample', 'full', 'none'],
                     help='sample: oracle on the first 50M pairs; full: on the whole config (minutes and tens of GB at C3)')
     ap.add_argument('--weak', action='store_true', help='N>1: weak scaling (a full --config shard per rank) instead of strong')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='N=1: after the timed steps, write what the last timed step returned as DIR/<name>.npy '
+                         '(float64; the edge list as a fixed, seeded sample when it is longer than {} edges)'.format(
+                             DUMP_EDGES))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
 
 
 def ncu_traffic(cfg, kernel):
@@ -306,6 +316,26 @@ def _wrap64(v):
     return int(v) & 0xffffffffffffffff
 
 
+def dump_outputs(out_dir, res):
+    """Write the edge result HotPath.run returned (the views are overwritten by the next run, so call this before it)
+    as out_dir/<name>.npy, all float64 (the int32 ids are exact in it).  An edge list longer than DUMP_EDGES is written
+    as the same seeded sample of positions on every run, with those positions in edge_index.npy."""
+    n = int(res['n_edges'])
+    out = {k: np.array([res[k]], dtype=np.float64) for k in ('n_accepted', 'n_kept', 'n_edges')}
+    out['scl'] = res['scl'][:1].cpu().numpy().astype(np.float64)
+    out['newidx'] = res['newidx'].cpu().numpy().astype(np.float64)
+    idx = np.arange(n) if n <= DUMP_EDGES else np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_EDGES,
+                                                                                               replace=False))
+    for k in ('u', 'v', 'w'):
+        out[k] = res[k][:n].cpu().numpy()[idx].astype(np.float64)
+    out['edge_index'] = idx.astype(np.float64)
+    total = sum(a.nbytes for a in out.values())
+    assert total <= 64 << 20, 'outputs to dump take {} B'.format(total)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
+
+
 # ---------------------------------------------------------------------------------------------------------------
 # N = 1
 # ---------------------------------------------------------------------------------------------------------------
@@ -350,8 +380,9 @@ def spmv_point(dev, torch, peak, rows, nnz, reps=20, seed=1005, compare=True):
     return out
 
 
-def run_single_gpu(work, args, torch, dev, local_rank, steps, warmup, want_cpu, parity_mode):
-    """Everything measured on one config on one GPU; returns the fields of a bench line."""
+def run_single_gpu(work, args, torch, dev, local_rank, steps, warmup, want_cpu, parity_mode, dump_dir=None):
+    """Everything measured on one config on one GPU; returns the fields of a bench line.  With dump_dir, what the last
+    timed step returned is written there (dump_outputs)."""
     from bin3c_b200 import bam_io
     from bin3c_b200.pipeline import HotPath
     P, N = work.P, work.N
@@ -401,6 +432,8 @@ def run_single_gpu(work, args, torch, dev, local_rank, steps, warmup, want_cpu, 
     digest = {'map': _wrap64(dg['map']), 'mask': _wrap64(dg['mask']), 'edges': _wrap64(dg['edges']),
               'map_weight': dg['weight'], 'nnz_full': dg['nnz'], 'n_edges': dg['n_edges'], 'n_iter': kr['n_iter'],
               'x_sum': dg['x_sum'], 'w_sum': dg['w_sum']}
+    if dump_dir:
+        dump_outputs(dump_dir, res)
 
     # ---- end-to-end arm: pinned host records in, host edge list out ------------------------------------
     # The records cross PCIe in the narrowest layout the reference table allows: the pairs whose mates lie on one
@@ -541,7 +574,8 @@ def main_single(args, local_rank):
     cfg = args.config or 'C3'
     work = Workload(cfg, args.scale)
     want_cpu = not args.no_cpu_baseline
-    head = run_single_gpu(work, args, torch, dev, local_rank, args.steps, args.warmup, want_cpu, args.parity)
+    head = run_single_gpu(work, args, torch, dev, local_rank, args.steps, args.warmup, want_cpu, args.parity,
+                          dump_dir=args.dump_outputs)
     del work
     torch.cuda.empty_cache()
     line = {'metric': METRIC, 'metric_note': METRIC_NOTE, 'value': head.pop('value'), 'unit': UNIT, 'n_gpus': 1,
@@ -807,6 +841,8 @@ def main():
     rank = int(os.environ.get('RANK', 0))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
+    if args.dump_outputs and (args.impl == 'reference' or world > 1):
+        raise SystemExit('--dump-outputs is for --impl ours on one GPU')
 
     if args.impl == 'reference':
         run_reference(args, rank)

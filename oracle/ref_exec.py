@@ -2,11 +2,12 @@
 TEST INFRASTRUCTURE -- NOT PRODUCT CODE.
 
 Runs the reference's own hot-path functions (cerebis/bin3C, Python 2.7) verbatim under
-Python 3 by exec'ing line ranges of the source where it lies under /root/reference.
-No reference source is copied into this repository.  This only works in the build
-container (the GPU box has no /root/reference); it is used by
-tests/golden/make_golden.py to produce the committed golden vectors that pin
-oracle/oracle.py, and by the "pinning" tests when the reference tree is present.
+Python 3 by exec'ing line ranges of its source, from a checkout of the reference at
+$BIN3C_REFERENCE (default oracle/_ref/, which git ignores): cerebis/bin3C at commit
+76ad2a9, with its Infomap binary built at external/Infomap.  No reference source is
+committed to this repository.  It is used by tests/golden/make_golden*.py to produce
+the committed golden vectors that pin oracle/oracle.py, and by the "pinning" tests,
+which skip when no reference checkout is present.
 
 Shims (SURVEY.md section 8c): np.int/np.float/np.bool aliases, xrange = range, and a
 `.H` property on SciPy sparse classes (removed from SciPy >= 1.14) used by
@@ -19,7 +20,7 @@ import textwrap
 import numpy as np
 import scipy.sparse as scisp
 
-REFERENCE_ROOT = os.environ.get('BIN3C_REFERENCE', '/root/reference')
+REFERENCE_ROOT = os.environ.get('BIN3C_REFERENCE', os.path.join(os.path.dirname(os.path.abspath(__file__)), '_ref'))
 
 # (file, first line, last line) of each function executed verbatim
 SLICES = {

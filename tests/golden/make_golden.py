@@ -1,8 +1,8 @@
 """
 Generate the golden vectors under tests/golden/ by running the REFERENCE's own functions
-(exec'd verbatim from /root/reference by oracle/ref_exec.py) on seeded synthetic inputs.
+(exec'd verbatim from a reference checkout by oracle/ref_exec.py) on seeded synthetic inputs.
 
-Run in the build container only:   python tests/golden/make_golden.py
+With a reference checkout (see oracle/ref_exec.py):   python tests/golden/make_golden.py
 
 What is reference-verbatim: Sparse2DAccumulator (+get_coo), max_offdiag, kr_biostochastic
 (+is_hermitian), compress  (sparse_utils.py:227-266, 269-281, 90-224, 284-314).

@@ -4,7 +4,7 @@ under Python 3 (oracle/ref_exec.run_bin_map) on a fake BAM of duck-typed alignme
 Sparse2DAccumulator, ExtentGrouping and find_nearest_jit.  Three filter settings (MAPQ only, strong matcher,
 min_insert), each with the contig map, the binned extent map and the pair counters.  The alignment stream is stored
 as flat arrays so that tests can rebuild it (and write it as a real BAM file for the native reader).
-Run in the build container:  python tests/golden/make_golden_binmap.py
+With a reference checkout (see oracle/ref_exec.py):  python tests/golden/make_golden_binmap.py
 """
 import os
 import random

@@ -4,7 +4,7 @@ the reference's own code: SeqOrder / ContactMap / sparse_utils / cluster.to_grap
 (oracle/ref_exec.run_reference_path, as in make_golden_refpath.py), then nx.write_edgelist in the layout the pinned
 Python 2.7 / networkx 1.11 produce (12 significant digits) and the reference's own Infomap binary with the flags of
 cluster.py:182-185.  Nothing here comes from oracle/oracle.py.  The pair records are not stored: they are
-synth.make_config('C1') (deterministic).  Run in the build container (needs /root/reference, ~15 s):
+synth.make_config('C1') (deterministic).  Run with a reference checkout (see oracle/ref_exec.py; ~15 s):
     python tests/golden/make_golden_c1.py
 """
 import logging

@@ -1,8 +1,8 @@
 """
 Golden vectors for the extent map's bins: the reference's own ExtentGrouping class and find_nearest_jit, exec'd
-verbatim from /root/reference/mzd/contact_map.py:50-62, 116-156 under Python 3 (oracle/ref_exec.load_extent: np.int
+verbatim from the reference's mzd/contact_map.py:50-62, 116-156 under Python 3 (oracle/ref_exec.load_extent: np.int
 alias, tqdm stub, numba decorator dropped, and sequence lengths wrapped in an int whose `/` is Python 2's integer
-division), on seeded random sequence lengths.  Run in the build container:  python tests/golden/make_golden_extent.py
+division), on seeded random sequence lengths.  With a reference checkout (see oracle/ref_exec.py):  python tests/golden/make_golden_extent.py
 """
 import os
 import random

@@ -4,7 +4,7 @@ _compress_extent (contact_map.py:1001-1036, 1147-1165, 1197-1249) -- produced by
 exec'd verbatim under Python 3 (oracle/ref_exec.run_reference_path with bin_size): _bin_map over duck-typed alignment
 records builds seq_map and extent_map, set_primary_acceptance_mask masks some sequences, then get_extent_map is called
 for every mean type, with and without balancing.  Nothing here comes from oracle/oracle.py.
-Run in the build container:  python tests/golden/make_golden_extentmap.py
+With a reference checkout (see oracle/ref_exec.py):  python tests/golden/make_golden_extentmap.py
 """
 import os
 import sys

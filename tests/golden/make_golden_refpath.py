@@ -5,7 +5,7 @@ pysam/Biopython part replayed from the reference table), driven as bin3C.py does
 set_primary_acceptance_mask -> to_graph [prepare_seq_map(norm, bisto) -> _norm_seq, _bisto_seq (kr_biostochastic);
 get_subspace(marginalise=True, flatten=False) -> compress] -- on a synthetic community whose pair records are
 presented as duck-typed alignment records.  Nothing here comes from oracle/oracle.py.
-Run in the build container:  python tests/golden/make_golden_refpath.py
+With a reference checkout (see oracle/ref_exec.py):  python tests/golden/make_golden_refpath.py
 """
 import logging
 import os

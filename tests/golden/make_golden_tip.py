@@ -8,7 +8,7 @@ Golden vectors for the tip-based map (SURVEY.md 8f rank 4): the reference's own 
   * the whole path by the reference's own classes: _bin_map -> set_primary_acceptance_mask -> to_graph
     [prepare_seq_map(norm, bisto) with fast_norm_tipbased_bysite, get_subspace(marginalise=True)]: mask, scale factors,
     processed tensor, graph edges; plus get_subspace(flatten=True).
-Run in the build container:  python tests/golden/make_golden_tip.py
+With a reference checkout (see oracle/ref_exec.py):  python tests/golden/make_golden_tip.py
 """
 import os
 import random

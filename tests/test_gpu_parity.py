@@ -966,6 +966,41 @@ def test_cuda_path_vs_whole_reference_path(dev):
     assert _relerr(pm.data[o1], g['bal_data'][o2]) <= REL_TOL
 
 
+def test_contact_map_mask_rules_against_the_reference_mask(dev):
+    """
+    The acceptance-mask rules of ContactMap.set_primary_acceptance_mask (contact_map.py:856-909, Q5) on the reference's
+    own path (refpath.npz): the mask is cached unless `update`; updated masks follow oracle.acceptance_mask on the
+    reference's contact matrix; falsy thresholds fall back to the instance's and give the reference's stored mask
+    again.  SeqOrder under that mask accepts exactly the reference's accepted contigs, in order, at the front.
+    """
+    import os
+    from oracle import oracle
+    from bin3c_b200.contact_map import ContactMap, PairRecords
+    with np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'refpath.npz')) as z:
+        g = {k: z[k] for k in z.files}
+    min_len, min_sig = int(g['min_len']), int(g['min_sig'])
+    cm = ContactMap(PairRecords(g['lengths'], g['sites'], g['records']), ['synthetic'], None, None, min_mapq=60,
+                    min_len=min_len, min_sig=min_sig, random_seed=1)
+    want = g['mask'].astype(bool)
+    n = len(want)
+    seq_len = g['lengths'][(g['lengths'] >= min_len) & (g['sites'] >= 0)]
+    sm = sp.coo_matrix((g['map_data'], (g['map_row'], g['map_col'])), shape=(n, n))
+    assert len(seq_len) == n
+    assert np.array_equal(cm.get_primary_acceptance_mask(), want)
+    cm.set_primary_acceptance_mask(min_len=5000, min_sig=20)                 # no update: the cached mask stays
+    assert np.array_equal(cm.get_primary_acceptance_mask(), want)
+    for ml, ms in ((5000, 20), (2000, 1), (1000, 50)):
+        cm.set_primary_acceptance_mask(min_len=ml, min_sig=ms, update=True)
+        assert np.array_equal(cm.get_primary_acceptance_mask(), oracle.acceptance_mask(seq_len, sm, ml, ms))
+    cm.set_primary_acceptance_mask(min_len=0, min_sig=0, update=True)       # falsy -> the instance's thresholds
+    assert np.array_equal(cm.get_primary_acceptance_mask(), want)
+    cm.order.set_mask_only(cm.get_primary_acceptance_mask())
+    assert np.array_equal(cm.order.mask_vector(), want) and cm.order.count_accepted() == int(want.sum())
+    assert np.array_equal(cm.order.accepted(), np.flatnonzero(want))
+    assert np.array_equal(cm.order.excluded(), np.flatnonzero(~want))
+    assert np.array_equal(np.sort(cm.order.order['pos'][want]), np.arange(int(want.sum())))
+
+
 def test_contact_map_from_bam_and_fasta_paths(dev, tmp_path):
     """
     The call bin3C.py mkmap makes (bin3C.py:148-158): ContactMap(BAM path, enzymes, FASTA path, min_insert, ...).  The

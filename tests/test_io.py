@@ -16,7 +16,7 @@ sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 import bam_writer                                   # noqa: E402
 from bin3c_b200 import bam_io                       # noqa: E402
-from oracle import oracle                           # noqa: E402
+from oracle import oracle, ref_exec                 # noqa: E402
 
 
 def random_alignments(rng, n_refs, n_templates, weird=True):
@@ -255,10 +255,11 @@ def test_cluster_write_edges_uses_the_native_writer(tmp_path):
     assert open(f).read() == '0 0 1.0\n0 2 0.25\n1 2 0.333333333333\n'
 
 
-INFOMAP = '/root/reference/external/Infomap'
+INFOMAP = os.path.join(ref_exec.REFERENCE_ROOT, 'external', 'Infomap')
 
 
-@pytest.mark.skipif(not os.access(INFOMAP, os.X_OK), reason='the reference tree (and its Infomap binary) is not present')
+@pytest.mark.skipif(not os.access(INFOMAP, os.X_OK), reason='no reference checkout with a built Infomap binary '
+                                                             '(oracle/_ref/ or $BIN3C_REFERENCE)')
 def test_infomap_partition_from_native_edge_file(tmp_path):
     """
     The hand-off itself: the reference's own Infomap binary, run with the reference's flags (cluster.py:182-185) on

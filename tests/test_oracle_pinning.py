@@ -1,8 +1,9 @@
 """
-Live pinning: where the reference tree is present (the build container), run its own
-functions verbatim (oracle/ref_exec.py) beside the oracle restatement on fresh seeded
-inputs.  Skipped on the GPU box, which has no /root/reference; the committed golden
-vectors (tests/test_oracle.py) carry the same check there.
+Live pinning: where a checkout of the reference is present (oracle/_ref/ or
+$BIN3C_REFERENCE, see oracle/ref_exec.py), run its own functions verbatim beside the
+oracle restatement on fresh seeded inputs (the tests marked needs_reference; skipped
+without one).  The committed golden vectors carry the same checks without a checkout:
+tests/test_oracle.py, and the tests at the end of this module.
 """
 import numpy as np
 import pytest
@@ -11,7 +12,7 @@ import scipy.sparse as sp
 from bin3c_b200 import synth
 from oracle import oracle, ref_exec
 
-pytestmark = pytest.mark.skipif(not ref_exec.available(), reason='reference tree not present')
+needs_reference = pytest.mark.skipif(not ref_exec.available(), reason='reference tree not present')
 
 
 @pytest.fixture(scope='module')
@@ -19,6 +20,7 @@ def fns():
     return ref_exec.load()
 
 
+@needs_reference
 @pytest.mark.parametrize('seed,n,p', [(101, 120, 4000), (102, 700, 25000), (103, 64, 300)])
 def test_reference_functions_vs_oracle(fns, seed, n, p):
     com = synth.make_community(n_genomes=3, n_contigs=n, n_pairs=p, seed=seed)
@@ -53,6 +55,7 @@ def test_reference_functions_vs_oracle(fns, seed, n, p):
         assert rc.shape == oc.shape and abs(rc - oc).max() == 0
 
 
+@needs_reference
 def test_reference_extent_grouping_vs_oracle():
     """The reference's ExtentGrouping class and find_nearest_jit, exec'd live (Python 2 division shimmed)."""
     import random
@@ -70,6 +73,7 @@ def test_reference_extent_grouping_vs_oracle():
                 assert int(find_nearest(np.asarray(r.map[k]), x)) == oracle.find_nearest(o['map'][k], x)
 
 
+@needs_reference
 def test_reference_bin_map_loop_vs_oracle():
     """The reference's _bin_map, exec'd live on a fresh random alignment stream, against the oracle's loop."""
     import os
@@ -105,6 +109,7 @@ def test_reference_bin_map_loop_vs_oracle():
             assert np.array_equal(got.data, want.data)
 
 
+@needs_reference
 def test_reference_to_graph_vs_oracle_edges(tmp_path):
     """
     The reference's to_graph (cluster.py:278-325), exec'd on the compressed balanced map of a synthetic community:
@@ -141,6 +146,7 @@ def test_reference_to_graph_vs_oracle_edges(tmp_path):
     assert open(f_nx).read() == open(f_b3).read()
 
 
+@needs_reference
 def test_whole_reference_path_vs_oracle():
     """The reference's ContactMap and SeqOrder classes exec'd live and driven end to end (oracle/ref_exec.py:
     run_reference_path), against oracle.run_path on a fresh community, with an extent map on the side."""
@@ -168,6 +174,7 @@ def test_whole_reference_path_vs_oracle():
     assert res['extent_map'].shape[0] == res['cm'].grouping.total_bins and res['extent_map'].sum() > 0
 
 
+@needs_reference
 def test_reference_seqorder_and_mask_rules_vs_product_host_logic():
     """
     The product's host-side SeqOrder (pure NumPy, no GPU) beside the reference's SeqOrder class on random masks, and
@@ -216,6 +223,7 @@ def test_reference_seqorder_and_mask_rules_vs_product_host_logic():
     assert np.array_equal(cm.get_primary_acceptance_mask(), first)
 
 
+@needs_reference
 def test_infomap_partition_reference_graph_vs_product_edge_list(tmp_path):
     """
     North-star: "the resulting Infomap clustering is identical".  The reference's graph (its own to_graph on its own
@@ -278,11 +286,12 @@ def _read_edge_file_gz(path):
     return np.array(u), np.array(v), np.array(w)
 
 
+@needs_reference
 def test_infomap_partition_of_gpu_edge_file(tmp_path):
     """
     North-star bar 3 on CUDA OUTPUT: tests/golden/c1_gpu.edges.gz and c1_gpu_py2.edges.gz are the edge files the CUDA
     path wrote on a B200 for BASELINE config 1 at full size (tests/test_gpu_configs.py::
-    test_c1_full_size_against_the_reference_own_output leaves them in gpurun_out/; committed unchanged, gzip'd).
+    test_c1_full_size_against_the_reference_own_output checks that it still writes them; committed gzip'd).
     They hold the reference's own edges (c1full.npz: the reference's classes exec'd on the same 1M pairs) to 1e-9,
     and the reference's Infomap binary, run here with the flags of cluster.py:182-185, returns for both the partition it
     returns for the reference's own graph file (stored in c1full.npz by make_golden_c1.py).
@@ -320,6 +329,7 @@ def test_infomap_partition_of_gpu_edge_file(tmp_path):
         assert np.array_equal(node, want[0]) and np.array_equal(label, want[1]), name
 
 
+@needs_reference
 def test_reference_tip_based_path_vs_oracle():
     """The tip-based map (SURVEY.md 8f rank 4), live: the reference's _bin_map with tip_size, its Sparse4DAccumulator and
     4-D functions over SparseShim, and its ContactMap class driven to the graph, beside the oracle on a fresh stream."""
@@ -351,3 +361,73 @@ def test_reference_tip_based_path_vs_oracle():
         e = sorted((min(u, v), max(u, v), d['weight']) for u, v, d in path['graph'].edges(data=True))
         assert [x[0] for x in e] == mine['u'].tolist() and [x[1] for x in e] == mine['v'].tolist()
         assert np.max(np.abs(np.array([x[2] for x in e]) - mine['w']) / np.abs(mine['w'])) <= 1e-12
+
+
+# ---- the same comparisons against outputs of the reference stored under tests/golden (no reference checkout) ----
+
+def _refpath_and_oracle():
+    """tests/golden/refpath.npz (the reference's own path, make_golden_refpath.py) and oracle.run_path on its inputs."""
+    from conftest import load_golden
+    g = load_golden('refpath')
+    keep = (g['lengths'] >= int(g['min_len'])) & (g['sites'] >= 0)
+    lut = np.where(keep, np.cumsum(keep) - 1, -1).astype(np.int32)
+    ti, tj, ok = synth.unpack_pairs(g['records'])
+    ref = oracle.run_path(ti, tj, ok, lut, g['lengths'][keep], g['sites'][keep], min_len=int(g['min_len']),
+                          min_sig=int(g['min_sig']))
+    return g, ref
+
+
+def test_stored_reference_graph_weights_are_its_mirrored_entries(tmp_path):
+    """
+    The graph the reference's to_graph built (refpath.npz): its scale is exactly the oracle's 1/max of the compressed
+    balanced map (Q8), and every weight is the reference's own balanced map at the mirrored (lower) position times that
+    scale -- the last of the two entries it adds wins (Q9).  The edge file networkx writes from that graph equals the
+    native writer's on the graph's own weights.
+    """
+    nx = pytest.importorskip('networkx')
+    from bin3c_b200 import bam_io
+    g, ref = _refpath_and_oracle()
+    n = len(g['mask'])
+    acc = np.flatnonzero(g['mask'])
+    sub = sp.coo_matrix((g['bal_data'], (g['bal_row'], g['bal_col'])), shape=(n, n)).tocsr()[acc][:, acc]
+    assert ref['scl'] == 1.0 / sub.max()
+    assert g['edge_w'].max() == ref['w'].max()
+    u, v, w = g['edge_u'], g['edge_v'], g['edge_w']
+    assert np.array_equal(w, np.asarray(sub[v, u]).ravel() * ref['scl'])
+    graph = nx.Graph()
+    for a, b, c in zip(u, v, w):
+        graph.add_edge(int(a), int(b), weight=float(c))
+    f_nx, f_b3 = str(tmp_path / 'nx.edges'), str(tmp_path / 'b3.edges')
+    nx.write_edgelist(graph, f_nx, data=['weight'], delimiter=' ')
+    e = list(graph.edges(data='weight'))
+    bam_io.write_edges([a for a, _, _ in e], [b for _, b, _ in e], [c for _, _, c in e], f_b3)
+    assert open(f_nx).read() == open(f_b3).read()
+
+
+def test_stored_reference_edge_file_equals_the_native_writers(tmp_path):
+    """The reference's graph (refpath.npz) in the 12-significant-digit layout its pinned Python 2.7 / networkx 1.11
+    write, and the oracle's edge list written by the native writer in that layout: byte-identical files, so Infomap
+    reads the same graph from both."""
+    from bin3c_b200 import bam_io
+    g, ref = _refpath_and_oracle()
+    f = str(tmp_path / 'cm_graph.edges')
+    bam_io.write_edges(ref['u'], ref['v'], ref['w'], f, float_style=bam_io.FLOAT_STR12)
+    assert open(f).read() == oracle.edge_lines(g['edge_u'], g['edge_v'], g['edge_w'], py2=True)
+
+
+def test_gpu_edge_files_hold_the_reference_edges():
+    """tests/golden/c1_gpu.edges.gz and c1_gpu_py2.edges.gz, the edge files the CUDA path wrote on a B200 for BASELINE
+    config 1, hold the reference's own edges (c1full.npz) to 1e-9; in the reference's 12-digit layout the GPU file is
+    the reference's file but for at most 3 lines."""
+    import gzip
+    import os
+    from conftest import load_golden, GOLDEN_DIR
+    g = load_golden('c1full')
+    u, v, w = _read_edge_file_gz(os.path.join(GOLDEN_DIR, 'c1_gpu.edges.gz'))
+    assert np.array_equal(u, g['edge_u']) and np.array_equal(v, g['edge_v'])
+    assert np.max(np.abs(w - g['edge_w']) / np.abs(g['edge_w'])) <= 1e-9
+    with gzip.open(os.path.join(GOLDEN_DIR, 'c1_gpu_py2.edges.gz'), 'rt') as fh:
+        gpu_py2 = fh.read()
+    ref_py2 = oracle.edge_lines(g['edge_u'], g['edge_v'], g['edge_w'], py2=True)
+    differing = sum(1 for a, b in zip(gpu_py2.splitlines(), ref_py2.splitlines()) if a != b)
+    assert len(gpu_py2.splitlines()) == len(ref_py2.splitlines()) and differing <= 3, differing

@@ -3,7 +3,7 @@ BASELINE config 1 made real: the reference's OWN code (oracle/ref_exec.run_refer
 sparse_utils and cluster.to_graph exec'd verbatim under Python 3) on the synthetic C1 community (10 genomes, 2,000
 contigs, 1M Hi-C pairs), then nx.write_edgelist and the reference's Infomap binary with the reference's flags --
 timed stage by stage on this machine's CPU, beside the vectorised port (oracle.run_path) and with the two partitions
-compared.  Needs /root/reference (build container only; no GPU).
+compared.  Needs a reference checkout (see oracle/ref_exec.py); no GPU.
     python tools/reference_c1.py [--scale 1.0]
 """
 import argparse
