@@ -488,9 +488,11 @@ def compress_edges(csr, mask, want_sub=True, want_edges=True, scale=True, pool=N
         sub_indices = _alloc(pool, 'sub_indices', n_kept, torch.int32)
         sub_data = _alloc(pool, 'sub_data', n_kept, torch.float64)
     if want_edges:
-        eu = _alloc(pool, 'edge_u', n_edges, torch.int32)
-        ev = _alloc(pool, 'edge_v', n_edges, torch.int32)
-        ew = _alloc(pool, 'edge_w', n_edges, torch.float64)
+        # at least one element: a zero-length tensor (or view) reports a null address, which the fused fill refuses as
+        # missing edge arrays; a block or a matrix without edges gets zero-length views of real buffers
+        eu = _alloc(pool, 'edge_u', max(n_edges, 1), torch.int32)
+        ev = _alloc(pool, 'edge_v', max(n_edges, 1), torch.int32)
+        ew = _alloc(pool, 'edge_w', max(n_edges, 1), torch.float64)
     scl = _alloc(pool, 'scl', 1, torch.float64)
     if fused:
         check(lib.b3c_edges_fill(n, csr.row_lo, nl, _ptr(csr.indptr), _ptr(csr.indices), _ptr(csr.data), _ptr(ws),
@@ -501,6 +503,8 @@ def compress_edges(csr, mask, want_sub=True, want_edges=True, scale=True, pool=N
                                     _ptr(sub_indptr), _ptr(sub_indices), _ptr(sub_data), _ptr(eu), _ptr(ev), _ptr(ew),
                                     _ptr(scl), _stream()))
     sub = DeviceCSR(n_acc, sub_indptr, sub_indices, sub_data) if want_sub else None
+    if want_edges:
+        eu, ev, ew = eu[:n_edges], ev[:n_edges], ew[:n_edges]
     return dict(n_accepted=n_acc, n_kept=n_kept, n_edges=n_edges, sub=sub, u=eu, v=ev, w=ew, scl=scl, newidx=newidx)
 
 
