@@ -17,6 +17,7 @@ B3C_ERR_CAPACITY = -3
 B3C_ERR_NOCONV = -4
 B3C_ERR_NAN = -5
 B3C_ERR_TIE = -6
+B3C_ERR_FORMAT = -7
 
 
 class B3CError(RuntimeError):
@@ -96,6 +97,10 @@ SIGNATURES = {
     'b3c_extent_norm': (C.c_int, [_i32, _i32, _p, _p, _p, _p, _i32, _p, _p]),
     'b3c_synth_pairs': (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _i32, _i32, _i32, _f64, _f64, _f64, _f64, C.c_uint64,
                                   C.c_uint64, _i64, _p, _p]),
+    'b3c_bamdec_workspace_bytes': (_i64, [_i32, _i32]),
+    'b3c_bamdec_begin': (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _i32, _i64, _p]),
+    'b3c_bamdec_slab': (C.c_int, [_p, _p, _p, _i32, _i64, _i64, _p, _i64, _p, _i64, _i32, _p, _i64, _pi64, _p]),
+    'b3c_bamdec_stats': (C.c_int, [_p, _pi64, _i32, _p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():
@@ -122,6 +127,8 @@ def check(rc):
         raise AssertionError(msg)                   # the reference asserts on bad arguments
     if rc == B3C_ERR_TIE:
         raise ValueError(msg)                       # np.amin of an empty selection (Q13)
+    if rc == B3C_ERR_FORMAT:
+        raise ValueError(msg)                       # malformed BAM file: what the host reader raises for it
     if rc in (B3C_ERR_NOCONV, B3C_ERR_NAN):
         raise RuntimeError(msg)                     # sparse_utils.py:193,214
     raise B3CError('b3c status {}: {}'.format(rc, msg))

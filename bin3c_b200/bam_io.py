@@ -25,6 +25,8 @@ B3C_IO_ERR_OPEN = -2
 B3C_IO_ERR_FORMAT = -3
 B3C_IO_ERR_SORT = -4
 
+DEFAULT_SLAB_BYTES = 256 << 20    # compressed bytes per slab of the device decoder
+
 FLOAT_REPR = 0       # Python 3 str(float) == repr(float)
 FLOAT_STR12 = 1      # Python 2.7 str(float): '%.12g' (+ '.0'), what the reference's pinned interpreter prints
 
@@ -47,6 +49,8 @@ SIGNATURES = {
     'b3c_bam_ref_name': (C.c_char_p, [_p, _i32]),
     'b3c_bam_ref_lengths': (_i64, [_p, _p, _i32]),
     'b3c_bam_header_text': (_i64, [_p, _p, _i64]),
+    'b3c_bam_data_offset': (_i64, [_p]),
+    'b3c_bgzf_scan': (_i64, [_p, _i64, _i32, _p, _p, _p, _i64, _p]),
     'b3c_bam_set_filter': (C.c_int, [_p, _i32, _i32, _i32, _p, _i32]),
     'b3c_bam_read_pairs': (_i64, [_p, _p, _i64]),
     'b3c_bam_set_extent': (C.c_int, [_p, _p, _i32, _p, _p, _p, _i32]),
@@ -195,7 +199,7 @@ class BamPairReader(object):
 
 
 def pair_records_from_bam(path, sites=None, min_mapq=60, strong=None, min_insert=None, min_len=None, threads=0,
-                          bin_size=None, tip_size=None):
+                          bin_size=None, tip_size=None, device=False, slab_bytes=DEFAULT_SLAB_BYTES, slab_blocks=None):
     """
     BAM file -> (PairRecords, stats): the object `ContactMap(bam_file=...)` takes in this package.
 
@@ -206,8 +210,18 @@ def pair_records_from_bam(path, sites=None, min_mapq=60, strong=None, min_insert
     :param tip_size: tip-based map (contact_map.py:631-670): records carry doubled ids 2 * tid + tip and
                   PairRecords.tip10 the same-sequence (tail, head) pairs; needs `min_len` like min_insert; `sites`
                   may then be an (n_refs, 2) array of (head, tail) site counts (seq_utils.py:146-158).
+    :param device: decode on the GPU (bin3c_b200/csrc/bamdec.cu): the records come back as a CUDA uint64 tensor
+                  with the values, order and stats of the host reader.  Only compressed bytes cross PCIe.  Contig-map
+                  records only: with bin_size or tip_size it raises NotImplementedError.
+    :param slab_bytes, slab_blocks: the device decoder reads the file in slabs of whole BGZF blocks, about slab_bytes
+                  compressed bytes and at most slab_blocks blocks (default 65536) each
     """
     from .contact_map import PairRecords
+    if device:
+        if bin_size or tip_size:
+            raise NotImplementedError('extent and tip records are not decoded on the GPU: read this BAM file with the '
+                                      'host reader (device=False)')
+        return _pair_records_on_device(path, sites, min_mapq, strong, min_insert, min_len, slab_bytes, slab_blocks)
     with BamPairReader(path, threads=threads) as bam:
         s = np.ones(bam.n_refs, dtype=np.int64) if sites is None else np.asarray(sites, dtype=np.int64)
         assert len(s) == bam.n_refs, 'one site count per BAM reference'
@@ -261,6 +275,148 @@ def pair_records_from_bam(path, sites=None, min_mapq=60, strong=None, min_insert
                     not_tip=stats['not_tip'])
         return PairRecords(bam.lengths, s, records, references=bam.references, extent_records=extent, meta=meta,
                            tip10=tip10), stats
+
+
+def _pair_records_on_device(path, sites, min_mapq, strong, min_insert, min_len, slab_bytes, slab_blocks):
+    """
+    pair_records_from_bam(device=True).  One host thread reads the file into two pinned slabs and lists each slab's
+    BGZF blocks (b3c_bgzf_scan) while the device decodes the previous slab (include/bin3c_b200.h: b3c_bamdec_*); each
+    slab goes to the device with one asynchronous copy, and the record tensor grows as slabs finish.
+    """
+    import queue
+    import threading
+    import torch
+    from . import _cabi
+    from .contact_map import PairRecords
+    if not torch.cuda.is_available():
+        raise RuntimeError('pair_records_from_bam(device=True) needs a CUDA device; the host reader is device=False')
+    with BamPairReader(path, threads=1) as bam:                 # header, sort order, reference table
+        references, lengths = bam.references, bam.lengths.copy()
+        data_offset = int(check(lib.b3c_bam_data_offset(bam._h)))
+    n_refs = len(references)
+    s = np.ones(n_refs, dtype=np.int64) if sites is None else np.asarray(sites, dtype=np.int64)
+    assert len(s) == n_refs, 'one site count per BAM reference'
+    tid2idx = None
+    if min_insert:
+        assert min_len is not None, 'min_insert needs min_len'
+        keep = (lengths >= min_len) & ((s >= 0) if s.ndim == 1 else (s >= 0).all(axis=1))
+        tid2idx = np.where(keep, np.cumsum(keep) - 1, -1).astype(np.int32)
+    slab_bytes = max(int(slab_bytes), 1)
+    max_blocks = int(slab_blocks) if slab_blocks else 1 << 16
+    assert max_blocks >= 1, 'slab_blocks must be positive'
+    cap = slab_bytes + 65536                                    # always holds one whole block (BSIZE < 2^16)
+
+    dev = torch.device('cuda', torch.cuda.current_device())
+    stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    ws = torch.empty(int(_cabi.lib.b3c_bamdec_workspace_bytes(max_blocks, n_refs)), dtype=torch.uint8, device=dev)
+    d_tid = torch.from_numpy(tid2idx).to(dev) if tid2idx is not None else None
+    _cabi.check(_cabi.lib.b3c_bamdec_begin(ws.data_ptr(), ws.numel(), int(min_mapq), int(strong or 0),
+                                           int(min_insert or 0), d_tid.data_ptr() if d_tid is not None else None,
+                                           n_refs, data_offset, stream))
+
+    pinned = [torch.empty(cap, dtype=torch.uint8, pin_memory=True) for _ in range(2)]
+    free, ready = queue.Queue(), queue.Queue()
+    for k in range(2):
+        free.put(k)
+
+    def read_slabs():
+        try:
+            left = np.empty(0, dtype=np.uint8)
+            eof = False
+            with open(path, 'rb') as f:
+                while True:
+                    k = free.get()
+                    if k is None:
+                        return
+                    a = pinned[k].numpy()
+                    n = len(left)
+                    a[:n] = left
+                    while n < cap and not eof:
+                        m = f.readinto(memoryview(a)[n:cap])
+                        eof = not m
+                        n += m or 0
+                    offs = np.empty(max_blocks, dtype=np.int64)
+                    bsz = np.empty(max_blocks, dtype=np.int32)
+                    isz = np.empty(max_blocks, dtype=np.int32)
+                    used = np.zeros(1, dtype=np.int64)
+                    nb = lib.b3c_bgzf_scan(a.ctypes.data, n, 1 if eof else 0, offs.ctypes.data, bsz.ctypes.data,
+                                           isz.ctypes.data, max_blocks, used.ctypes.data)
+                    if nb < 0:
+                        ready.put(('error', nb, '{}: {}'.format(path, last_error())))
+                        return
+                    c = int(used[0])
+                    left = a[c:n].copy()
+                    last = eof and c == n
+                    ready.put((k, int(nb), c, offs[:nb], bsz[:nb], isz[:nb], last))
+                    if last:
+                        return
+        except BaseException as e:                              # handed to the decoding thread
+            ready.put(('error', None, e))
+
+    reader = threading.Thread(target=read_slabs, name='bam-slab-reader', daemon=True)
+    reader.start()
+    d_comp = torch.empty(cap, dtype=torch.uint8, device=dev)
+    u_bufs = [None, None]
+    out = torch.empty(1 << 20, dtype=torch.uint64, device=dev)
+    n_out, stream_off, next_rec = 0, 0, data_offset
+    prev_u, prev_u0, repaired, n_slabs = None, 0, 0, 0
+    res = (C.c_int64 * 4)()
+    try:
+        while True:
+            item = ready.get()
+            if item[0] == 'error':
+                if item[1] is None:
+                    raise item[2]
+                raise ValueError(item[2])                       # the reader's status for a bad BGZF block
+            k, nb, c, offs, bsz, isz, last = item
+            tbl = np.empty((nb, 3), dtype=np.int64)
+            tbl[:, 0] = offs
+            tbl[:, 1] = bsz.astype(np.int64) | (isz.astype(np.int64) << 32)
+            u_off = np.cumsum(isz, dtype=np.int64)
+            tbl[:, 2] = u_off - isz
+            u_bytes = int(u_off[-1]) if nb else 0
+            carry = max(0, stream_off - next_rec)
+            slot = n_slabs & 1
+            need = carry + u_bytes
+            if u_bufs[slot] is None or u_bufs[slot].numel() < max(need, 1):
+                u_bufs[slot] = None
+                u_bufs[slot] = torch.empty(max(need + need // 4, 1 << 16), dtype=torch.uint8, device=dev)
+            u = u_bufs[slot]
+            d_carry = prev_u.data_ptr() + (next_rec - prev_u0) if carry else None
+            bound = need // 72 + 2
+            if out.numel() - n_out < bound:
+                grown = torch.empty(max(2 * out.numel(), n_out + bound), dtype=torch.uint64, device=dev)
+                grown[:n_out].copy_(out[:n_out])
+                out = grown
+            if c:
+                d_comp[:c].copy_(pinned[k][:c], non_blocking=True)
+            d_tbl = torch.from_numpy(tbl.reshape(-1)).pin_memory().to(dev, non_blocking=True) if nb else None
+            rc = _cabi.lib.b3c_bamdec_slab(ws.data_ptr(), d_comp.data_ptr(), d_tbl.data_ptr() if nb else None, nb,
+                                           stream_off, u_bytes, d_carry, carry, u.data_ptr(), u.numel(),
+                                           1 if last else 0, out.data_ptr() + 8 * n_out, out.numel() - n_out, res,
+                                           stream)
+            free.put(k)                                         # the slab call synchronised: the pinned slab is free
+            if rc == _cabi.B3C_ERR_FORMAT:
+                raise ValueError('{}: {}'.format(path, _cabi.last_error()))
+            _cabi.check(rc)
+            n_out += int(res[0])
+            prev_u, prev_u0 = u, stream_off - carry
+            next_rec = int(res[1])
+            repaired += int(res[2])
+            stream_off += u_bytes
+            n_slabs += 1
+            if last:
+                break
+    finally:
+        free.put(None)
+        reader.join()
+    st = np.zeros(8, dtype=np.int64)
+    _cabi.check(_cabi.lib.b3c_bamdec_stats(ws.data_ptr(), st.ctypes.data_as(C.POINTER(C.c_int64)), 8, stream))
+    stats = dict(zip(STAT_NAMES, st.tolist() + [0]))
+    meta = dict(min_mapq=min_mapq, strong=strong, min_insert=min_insert or None, min_len=min_len, bin_size=None,
+                short_insert=stats['short_insert'], tip_size=None, not_tip=0, gpu_decode=True, slabs=n_slabs,
+                repaired_blocks=repaired)
+    return PairRecords(lengths, s, out[:n_out], references=references, meta=meta), stats
 
 
 def records_bytes(n_refs):

@@ -187,15 +187,17 @@ class ContactMap(object):
 
     def __init__(self, bam_file, enzymes, seq_file, min_insert, min_mapq=0, min_len=0, min_sig=1, min_extent=0,
                  min_size=0, max_fold=None, random_seed=None, strong=None, bin_size=None, tip_size=None,
-                 precount=False):
+                 precount=False, gpu_decode=False):
 
         assert not (tip_size and bin_size), 'tip records and extent records do not combine in this build'
         if not isinstance(bam_file, PairRecords):
             # the call bin3C.py mkmap makes (bin3C.py:148-158): a BAM path and a FASTA path.  The BAM is decoded by
             # the native reader (libbin3c_io.so) with this map's matcher, insert filter and bins; the site counts come
             # from the FASTA (seq_sites.fasta_site_table), or from `seq_file` given as an array / dict / callable.
+            # gpu_decode=True decodes the BAM on the GPU instead (bam_io.pair_records_from_bam(device=True)): the
+            # same records, left on the device for the accumulation.
             bam_file = self._open_bam(bam_file, enzymes, seq_file, min_insert, min_mapq, min_len, strong, bin_size,
-                                      tip_size)
+                                      tip_size, gpu_decode=gpu_decode)
         meta = bam_file.meta
         if tip_size:
             assert meta is not None and meta.get('tip_size') == tip_size and meta.get('min_len') == min_len, \
@@ -290,7 +292,8 @@ class ContactMap(object):
         self.set_primary_acceptance_mask()
 
     @staticmethod
-    def _open_bam(path, enzymes, seq_file, min_insert, min_mapq, min_len, strong, bin_size, tip_size=None):
+    def _open_bam(path, enzymes, seq_file, min_insert, min_mapq, min_len, strong, bin_size, tip_size=None,
+                  gpu_decode=False):
         """BAM path -> PairRecords with this map's filters (contact_map.py:520-564: FASTA pass, header, reference table).
         `seq_file`: a FASTA path; or per-reference site counts as an array (one per BAM reference), a dict
         {reference name: sites} (absent = not in the FASTA), or a callable (name, length) -> sites."""
@@ -322,7 +325,7 @@ class ContactMap(object):
         if tip_size and sites.ndim == 1:
             sites = np.array([[v, v] if np.ndim(v) == 0 else list(v) for v in sites.tolist()], dtype=np.int64)
         rec, _ = bam_io.pair_records_from_bam(path, sites=sites, min_mapq=min_mapq, strong=strong, min_insert=min_insert,
-                                              min_len=min_len, bin_size=bin_size, tip_size=tip_size)
+                                              min_len=min_len, bin_size=bin_size, tip_size=tip_size, device=gpu_decode)
         return rec
 
     # ---- pickling: host containers only ------------------------------------------------------

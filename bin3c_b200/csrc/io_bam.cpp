@@ -89,6 +89,7 @@ struct b3c_bam {
     std::string text;
     std::vector<std::string> ref_names;
     std::vector<int64_t> ref_lens;
+    int64_t data_off = 0;                  // uncompressed stream offset of the first alignment record
     // filter
     int32_t min_mapq = 0, strong = 0, min_insert = 0;
     std::vector<int32_t> tid2idx;
@@ -362,6 +363,7 @@ int parse_header(b3c_bam *h, int require_queryname) {
     const uint8_t *p = take(h, 8, &part);
     if (!p || memcmp(p, "BAM\1", 4) != 0) return fail_format(h, "not a BAM file (bad magic)");
     const uint32_t l_text = rd32(p + 4);
+    int64_t off = 8 + (int64_t)l_text + 4;
     if (l_text) {
         p = take(h, l_text, &part);
         if (!p) return fail_format(h, "truncated BAM header");
@@ -383,7 +385,9 @@ int parse_header(b3c_bam *h, int require_queryname) {
         if (!p || l_name == 0) return fail_format(h, "truncated reference table");
         h->ref_names.emplace_back((const char *)p, strnlen((const char *)p, l_name));
         h->ref_lens.push_back((int32_t)rd32(p + l_name));
+        off += 4 + (int64_t)l_name + 4;
     }
+    h->data_off = off;
     if (require_queryname) {
         // bam.header['HD']['SO'] == 'queryname' (contact_map.py:537-538)
         bool ok = false;
@@ -573,6 +577,68 @@ int64_t b3c_bam_header_text(const b3c_bam *h, char *h_text, int64_t capacity) {
         memcpy(h_text, h->text.data(), m);
         h_text[m] = '\0';
     }
+    return n;
+}
+
+int64_t b3c_bam_data_offset(const b3c_bam *h) { return h ? h->data_off : B3C_IO_ERR_ARG; }
+
+int64_t b3c_bgzf_scan(const uint8_t *h_buf, int64_t n_bytes, int32_t at_eof, int64_t *h_offsets, int32_t *h_bsize,
+                      int32_t *h_isize, int64_t capacity, int64_t *h_consumed) {
+    if ((!h_buf && n_bytes > 0) || n_bytes < 0 || capacity < 0 || !h_consumed ||
+        (capacity > 0 && (!h_offsets || !h_bsize || !h_isize))) {
+        set_err("b3c_bgzf_scan: bad argument");
+        return B3C_IO_ERR_ARG;
+    }
+    // the checks of read_block, on a buffer: a block cut off by the end of the buffer ends the scan, and is an error
+    // only when the file ends there
+    int64_t o = 0, n = 0;
+    *h_consumed = 0;
+    while (n < capacity && o < n_bytes) {
+        const uint8_t *hd = h_buf + o;
+        const int64_t left = n_bytes - o;
+        if (left < 12) {
+            if (!at_eof) break;
+            set_err("not a BGZF file (bad gzip member header)");
+            return B3C_IO_ERR_FORMAT;
+        }
+        if (hd[0] != 0x1f || hd[1] != 0x8b || hd[2] != 8 || !(hd[3] & 4)) {
+            set_err("not a BGZF file (bad gzip member header)");
+            return B3C_IO_ERR_FORMAT;
+        }
+        const int xlen = rd16(hd + 10);
+        if (left < 12 + xlen) {
+            if (!at_eof) break;
+            set_err("truncated BGZF block");
+            return B3C_IO_ERR_FORMAT;
+        }
+        int bsize = -1;
+        for (int e = 0; e + 4 <= xlen;) {
+            const int slen = rd16(hd + 12 + e + 2);
+            if (hd[12 + e] == 'B' && hd[12 + e + 1] == 'C' && slen == 2 && e + 6 <= xlen) bsize = rd16(hd + 12 + e + 4);
+            e += 4 + slen;
+        }
+        const long payload = (long)bsize + 1 - 12 - xlen - 8;
+        if (bsize < 0 || payload < 0) {
+            set_err("not a BGZF file (no BC subfield)");
+            return B3C_IO_ERR_FORMAT;
+        }
+        if (left < (int64_t)bsize + 1) {
+            if (!at_eof) break;
+            set_err("truncated BGZF block");
+            return B3C_IO_ERR_FORMAT;
+        }
+        const uint32_t isize = rd32(hd + bsize + 1 - 4);
+        if (isize > 65536) {
+            set_err("corrupt BGZF block (ISIZE > 64 KiB)");
+            return B3C_IO_ERR_FORMAT;
+        }
+        h_offsets[n] = o;
+        h_bsize[n] = bsize;
+        h_isize[n] = (int32_t)isize;
+        ++n;
+        o += (int64_t)bsize + 1;
+    }
+    *h_consumed = o;
     return n;
 }
 

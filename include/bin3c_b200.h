@@ -41,7 +41,8 @@ typedef enum {
     B3C_ERR_CAPACITY = -3,   /* caller-supplied buffer or workspace too small           */
     B3C_ERR_NOCONV = -4,     /* KR: n_iter > max_iter (RuntimeError, sparse_utils.py:213) */
     B3C_ERR_NAN = -5,        /* KR: scale vector developed NaNs (sparse_utils.py:192)   */
-    B3C_ERR_TIE = -6         /* KR: max(ynew) == Delta exactly (ValueError, Q13, sparse_utils.py:179-181) */
+    B3C_ERR_TIE = -6,        /* KR: max(ynew) == Delta exactly (ValueError, Q13, sparse_utils.py:179-181) */
+    B3C_ERR_FORMAT = -7      /* BAM decoder: malformed file (ValueError, as the host reader raises)  */
 } b3c_status;
 
 int b3c_version(void);
@@ -425,6 +426,42 @@ int b3c_synth_pairs(const double *d_cum_w1, const double *d_cum_len, const int32
                     const int32_t *d_excl_tids, int32_t n_contigs, int32_t n_genomes, int32_t n_excl,
                     double p_same, double p_genome, double p_pass, double excl_end_frac, uint64_t seed,
                     uint64_t first, int64_t count, uint64_t *d_records, void *stream);
+
+/* ------------------------------------------------------------------------------------
+ * BAM decoding (the step before the path, on the device; bin3c_b200/csrc/bamdec.cu).  A name-sorted
+ * BAM file -> the packed pair records of the contig map, the same values in the same order as the host
+ * reader (include/bin3c_io.h: b3c_bam_read_pairs) writes, and the same counters.  The host parses the
+ * header (b3c_bam_open, b3c_bam_data_offset), reads the file in SLABS of whole BGZF blocks and lists each
+ * slab's blocks (b3c_bgzf_scan); the decoder inflates, checks ISIZE and CRC-32, finds the record
+ * boundaries, parses and pairs on the device.
+ *
+ *   workspace_bytes  decoder state, the tid -> index table and per-block scratch for up to max_blocks
+ *              blocks per slab
+ *   begin      once per file: matcher and insert filter as b3c_bam_set_filter (d_tid2idx: int32[n_refs],
+ *              device, may be NULL when min_insert <= 0; copied), data_offset = b3c_bam_data_offset
+ *   slab       one slab: d_comp = the slab's compressed bytes (device); d_blocks = int64[3 n_blocks]:
+ *              offset of the block in d_comp, BSIZE | ISIZE << 32, offset of the block's first inflated
+ *              byte from the slab's first (the exclusive sum of ISIZE); stream_offset = uncompressed stream
+ *              offset of the slab's first inflated byte (header blocks included); u_bytes = sum of ISIZE.
+ *              The previous slab may end inside a record: h_result[1] of the previous call is the stream
+ *              offset where that record starts, and the carry_bytes = stream_offset - h_result[1] bytes
+ *              before stream_offset (from the previous call's d_u) are passed as d_carry.  d_u receives the
+ *              carry and the inflated blocks (u_capacity >= carry_bytes + u_bytes); it must not overlap
+ *              d_carry.  Records go to d_out[0 .. h_result[0]); out_capacity >= (carry_bytes + u_bytes) / 72
+ *              + 2 always suffices.  `last` != 0 on the slab that ends the file.  Synchronises the stream
+ *              once.  h_result[4]: records written, stream offset of the first record not decoded,
+ *              blocks whose record boundary was repaired, informative records.  A malformed file ->
+ *              B3C_ERR_FORMAT; b3c_last_error() names the first error and its uncompressed stream offset.
+ *   stats      h_stats[0..7] = b3c_bam_stats indices 0-7 (synchronises)
+ * ------------------------------------------------------------------------------------ */
+int64_t b3c_bamdec_workspace_bytes(int32_t max_blocks, int32_t n_refs);
+int b3c_bamdec_begin(void *d_ws, int64_t ws_bytes, int32_t min_mapq, int32_t strong, int32_t min_insert,
+                     const int32_t *d_tid2idx, int32_t n_refs, int64_t data_offset, void *stream);
+int b3c_bamdec_slab(void *d_ws, const uint8_t *d_comp, const int64_t *d_blocks, int32_t n_blocks,
+                    int64_t stream_offset, int64_t u_bytes, const uint8_t *d_carry, int64_t carry_bytes,
+                    uint8_t *d_u, int64_t u_capacity, int32_t last, uint64_t *d_out, int64_t out_capacity,
+                    int64_t *h_result, void *stream);
+int b3c_bamdec_stats(const void *d_ws, int64_t *h_stats, int32_t n_stats, void *stream);
 
 #ifdef __cplusplus
 }

@@ -60,6 +60,18 @@ const char *b3c_bam_ref_name(const b3c_bam *bam, int32_t tid);
 int64_t b3c_bam_ref_lengths(const b3c_bam *bam, int64_t *h_lengths, int32_t capacity);
 int64_t b3c_bam_header_text(const b3c_bam *bam, char *h_text, int64_t capacity);   /* returns the full length */
 
+/* Uncompressed stream offset of the first alignment record (the end of the header parsed by b3c_bam_open). */
+int64_t b3c_bam_data_offset(const b3c_bam *bam);
+
+/* The BGZF block table of a host buffer that starts at a block: for each complete block, its offset in the buffer,
+ * BSIZE (the block's length minus one, from the BC extra subfield) and ISIZE (from the trailer).  Stops at `capacity`
+ * blocks or at the first block the buffer does not hold completely; *h_consumed = the bytes of the blocks listed (the
+ * next block starts there).  The header checks are those of the reader (gzip magic, the BC subfield, ISIZE <= 64 KiB)
+ * and fail with B3C_IO_ERR_FORMAT; a block cut off by the end of the buffer fails the same way when at_eof != 0 (the
+ * file ends there), and ends the scan otherwise.  Returns the number of blocks listed or a negative status. */
+int64_t b3c_bgzf_scan(const uint8_t *h_buf, int64_t n_bytes, int32_t at_eof, int64_t *h_offsets, int32_t *h_bsize,
+                      int32_t *h_isize, int64_t capacity, int64_t *h_consumed);
+
 /* Matcher and insert filter; call before the first read.
  *   min_mapq     r.mapping_quality >= min_mapq                         (_simple_match, :612-613)
  *   strong       > 0: also the 5'-end CIGAR op must be M with length >= strong; a record without
