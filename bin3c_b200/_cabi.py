@@ -101,6 +101,10 @@ SIGNATURES = {
     'b3c_bamdec_begin': (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _i32, _i64, _p]),
     'b3c_bamdec_slab': (C.c_int, [_p, _p, _p, _i32, _i64, _i64, _p, _i64, _p, _i64, _i32, _p, _i64, _pi64, _p]),
     'b3c_bamdec_stats': (C.c_int, [_p, _pi64, _i32, _p]),
+    'b3c_sites_workspace_bytes': (_i64, [_i64, _i32]),
+    'b3c_sites_begin': (C.c_int, [_p, _i64, _i64, _p, _p, _p, _i32, _i32, _p]),
+    'b3c_sites_slab': (C.c_int, [_p, _p, _i64, _p, _i64, _p, _i64, _pi64, _p]),
+    'b3c_sites_finish': (C.c_int, [_p, _p, _p, _i64, _pi64, _p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

@@ -187,7 +187,7 @@ class ContactMap(object):
 
     def __init__(self, bam_file, enzymes, seq_file, min_insert, min_mapq=0, min_len=0, min_sig=1, min_extent=0,
                  min_size=0, max_fold=None, random_seed=None, strong=None, bin_size=None, tip_size=None,
-                 precount=False, gpu_decode=False):
+                 precount=False, gpu_decode=False, gpu_sites=False):
 
         assert not (tip_size and bin_size), 'tip records and extent records do not combine in this build'
         if not isinstance(bam_file, PairRecords):
@@ -195,9 +195,10 @@ class ContactMap(object):
             # the native reader (libbin3c_io.so) with this map's matcher, insert filter and bins; the site counts come
             # from the FASTA (seq_sites.fasta_site_table), or from `seq_file` given as an array / dict / callable.
             # gpu_decode=True decodes the BAM on the GPU instead (bam_io.pair_records_from_bam(device=True)): the
-            # same records, left on the device for the accumulation.
+            # same records, left on the device for the accumulation.  gpu_sites=True counts the FASTA's sites on the
+            # GPU (seq_sites.fasta_site_table(device=True)): the same counts.
             bam_file = self._open_bam(bam_file, enzymes, seq_file, min_insert, min_mapq, min_len, strong, bin_size,
-                                      tip_size, gpu_decode=gpu_decode)
+                                      tip_size, gpu_decode=gpu_decode, gpu_sites=gpu_sites)
         meta = bam_file.meta
         if tip_size:
             assert meta is not None and meta.get('tip_size') == tip_size and meta.get('min_len') == min_len, \
@@ -293,7 +294,7 @@ class ContactMap(object):
 
     @staticmethod
     def _open_bam(path, enzymes, seq_file, min_insert, min_mapq, min_len, strong, bin_size, tip_size=None,
-                  gpu_decode=False):
+                  gpu_decode=False, gpu_sites=False):
         """BAM path -> PairRecords with this map's filters (contact_map.py:520-564: FASTA pass, header, reference table).
         `seq_file`: a FASTA path; or per-reference site counts as an array (one per BAM reference), a dict
         {reference name: sites} (absent = not in the FASTA), or a callable (name, length) -> sites."""
@@ -308,7 +309,7 @@ class ContactMap(object):
         elif isinstance(seq_file, (str, bytes, os.PathLike)):
             from .seq_sites import fasta_site_table
             logger.info('Analyzing sites...')
-            info = fasta_site_table(seq_file, enzymes, min_len or 0, tip_size=tip_size)
+            info = fasta_site_table(seq_file, enzymes, min_len or 0, tip_size=tip_size, device=gpu_sites)
             sites = np.full((len(names), 2) if tip_size else len(names), -1, dtype=np.int64)
             for n, (nm, ln) in enumerate(zip(names, lengths)):
                 fa = info.get(nm)

@@ -463,6 +463,41 @@ int b3c_bamdec_slab(void *d_ws, const uint8_t *d_comp, const int64_t *d_blocks, 
                     int64_t *h_result, void *stream);
 int b3c_bamdec_stats(const void *d_ws, int64_t *h_stats, int32_t n_stats, void *stream);
 
+/* ------------------------------------------------------------------------------------
+ * Restriction-site counts of a FASTA file (the other input of ContactMap's FASTA path, on the device;
+ * bin3c_b200/csrc/sites.cu, sites.cuh).  Per sequence: its length, its site count (or the head and tail
+ * site counts of a tip-based map) and the byte range of its name in a NAME ARENA: what
+ * seq_sites.fasta_site_table computes from the file read in text mode.  The host reads (and inflates) the
+ * file into slabs of up to slab_bytes bytes, cut anywhere; the device does everything else.
+ *
+ *   workspace_bytes  state, per-slab scratch for slabs of up to slab_bytes (<= B3C_SITES_MAX_SLAB) bytes,
+ *              and the saved first and last tip_size bases of the open sequence (tip_size 0: no tips)
+ *   begin      once per file: n_patterns distinct patterns (<= B3C_SITES_MAX_PATTERNS), pattern p =
+ *              h_lengths[p] (1..B3C_SITES_MAX_LEN) IUPAC masks (A 1, C 2, G 4, T 8, OR-ed) at
+ *              h_masks[p * B3C_SITES_MAX_LEN + i], counted h_weights[p] times; host arrays.  Synchronises.
+ *   slab       the next n_bytes (>= 1) bytes of the file at d_bytes (device).  d_seqs = int64[seq_capacity][5]
+ *              per-sequence table, d_names = the name arena (uint8[names_capacity]); both are kept from slab
+ *              to slab and may be moved to a larger allocation between calls (contents copied).  When they
+ *              are too small the call writes nothing, returns B3C_ERR_CAPACITY with h_result[0] = rows and
+ *              h_result[1] = name bytes needed, and the same slab is passed again.  A byte >= 0x80 in a
+ *              line that is not a header -> B3C_ERR_FORMAT (text-mode lengths count characters).
+ *              h_result[3]: sequences, name bytes, kept bases so far.  Synchronises the stream once.
+ *   finish     after the last slab: d_out = int64[out_rows][5] (out_rows >= sequences): per sequence its
+ *              length, name range [lo, hi) in the arena, sites (tip maps: head sites), tail sites (tip maps;
+ *              else 0).  h_result[3] as for slab.  Synchronises.
+ * ------------------------------------------------------------------------------------ */
+#define B3C_SITES_MAX_LEN 16
+#define B3C_SITES_MAX_PATTERNS 64
+#define B3C_SITES_MAX_SLAB (1LL << 30)
+int64_t b3c_sites_workspace_bytes(int64_t slab_bytes, int32_t tip_size);
+int b3c_sites_begin(void *d_ws, int64_t ws_bytes, int64_t slab_bytes, const uint8_t *h_masks,
+                    const int32_t *h_lengths, const int32_t *h_weights, int32_t n_patterns, int32_t tip_size,
+                    void *stream);
+int b3c_sites_slab(void *d_ws, const uint8_t *d_bytes, int64_t n_bytes, int64_t *d_seqs, int64_t seq_capacity,
+                   uint8_t *d_names, int64_t names_capacity, int64_t *h_result, void *stream);
+int b3c_sites_finish(void *d_ws, int64_t *d_seqs, int64_t *d_out, int64_t out_rows, int64_t *h_result,
+                     void *stream);
+
 #ifdef __cplusplus
 }
 #endif
