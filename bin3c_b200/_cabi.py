@@ -19,6 +19,8 @@ B3C_ERR_NAN = -5
 B3C_ERR_TIE = -6
 B3C_ERR_FORMAT = -7
 
+B3C_EDGES_MAX_LINE_BYTES = 49     # the longest line b3c_edges_text writes
+
 
 class B3CError(RuntimeError):
     """CUDA-side failure reported by the library."""
@@ -105,6 +107,8 @@ SIGNATURES = {
     'b3c_sites_begin': (C.c_int, [_p, _i64, _i64, _p, _p, _p, _i32, _i32, _p]),
     'b3c_sites_slab': (C.c_int, [_p, _p, _i64, _p, _i64, _p, _i64, _pi64, _p]),
     'b3c_sites_finish': (C.c_int, [_p, _p, _p, _i64, _pi64, _p]),
+    'b3c_edges_text_workspace_bytes': (_i64, [_i64]),
+    'b3c_edges_text': (C.c_int, [_p, _i64, _p, _p, _p, _i64, _i32, _i32, _p, _i64, _pi64, _p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

@@ -484,8 +484,21 @@ def format_weight(w, float_style=FLOAT_REPR):
     return buf.value.decode('ascii')
 
 
+def _is_cuda(x):
+    return bool(getattr(x, 'is_cuda', False))
+
+
 def write_edges(u, v, w, path, sep=' ', float_style=FLOAT_REPR, threads=0):
-    """One 'u v weight' line per edge, as nx.write_edgelist(g, path, data=['weight'], delimiter=sep)."""
+    """
+    One 'u v weight' line per edge, as nx.write_edgelist(g, path, data=['weight'], delimiter=sep).  Returns the bytes
+    written.  Host arrays are formatted by the host writer (b3c_edges_write_fmt, `threads` threads); when u, v and w
+    are all CUDA tensors (cluster.to_edges(..., device=True)) the lines are formatted on their device and only the
+    text crosses PCIe (_write_edges_on_device).  The file is the same byte for byte either way.
+    """
+    cuda = [_is_cuda(x) for x in (u, v, w)]
+    if any(cuda):
+        assert all(cuda), 'u, v and w must be all CUDA tensors or all host arrays'
+        return _write_edges_on_device(u, v, w, path, sep, float_style)
     u = np.ascontiguousarray(u, dtype=np.int32)
     v = np.ascontiguousarray(v, dtype=np.int32)
     w = np.ascontiguousarray(w, dtype=np.float64)
@@ -493,3 +506,81 @@ def write_edges(u, v, w, path, sep=' ', float_style=FLOAT_REPR, threads=0):
     assert isinstance(sep, str) and len(sep) == 1, 'single-character separator'
     return check(lib.b3c_edges_write_fmt(os.fsencode(path), u.ctypes.data, v.ctypes.data, w.ctypes.data, len(u),
                                          sep.encode('ascii'), int(float_style), int(threads)))
+
+
+DEFAULT_EDGE_CHUNK = 1 << 21      # edges per device formatting call (text buffers of 49 bytes per edge)
+
+
+def _write_edges_on_device(u, v, w, path, sep=' ', float_style=FLOAT_REPR, chunk_edges=DEFAULT_EDGE_CHUNK):
+    """
+    write_edges for CUDA tensors.  The device formats chunk_edges edges at a time into a text buffer
+    (include/bin3c_b200.h: b3c_edges_text); each chunk's text is copied into one of two pinned host slabs, and one
+    writer thread writes slab k to the file while the device formats chunk k + 1.  Returns the bytes written.
+    """
+    import queue
+    import threading
+    import torch
+    from . import _cabi
+    assert len(u) == len(v) == len(w)
+    assert isinstance(sep, str) and len(sep) == 1, 'single-character separator'
+    sep_byte = sep.encode('ascii')[0]
+    assert float_style in (FLOAT_REPR, FLOAT_STR12), 'float_style is FLOAT_REPR or FLOAT_STR12'
+    dev = u.device
+    assert v.device == dev and w.device == dev, 'u, v and w must be on one device'
+    chunk = max(1, int(chunk_edges))
+    n = len(u)
+    with open(path, 'wb') as f, torch.cuda.device(dev):
+        if n == 0:
+            return 0
+        u = u.reshape(-1).to(torch.int32).contiguous()
+        v = v.reshape(-1).to(torch.int32).contiguous()
+        w = w.reshape(-1).to(torch.float64).contiguous()
+        chunk = min(chunk, n)
+        cap = _cabi.B3C_EDGES_MAX_LINE_BYTES * chunk
+        stream = torch.cuda.current_stream()
+        ws = torch.empty(int(_cabi.lib.b3c_edges_text_workspace_bytes(chunk)), dtype=torch.uint8, device=dev)
+        text = torch.empty(cap, dtype=torch.uint8, device=dev)
+        slabs = [torch.empty(cap, dtype=torch.uint8, pin_memory=True) for _ in range(2 if n > chunk else 1)]
+        free, ready = queue.Queue(), queue.Queue()
+        for k in range(len(slabs)):
+            free.put(k)
+        failed = []
+
+        def write_slabs():
+            try:
+                while True:
+                    item = ready.get()
+                    if item is None:
+                        return
+                    k, nb = item
+                    f.write(memoryview(slabs[k].numpy())[:nb])
+                    free.put(k)
+            except BaseException as e:                          # handed to the formatting thread
+                failed.append(e)
+                free.put(None)
+
+        writer = threading.Thread(target=write_slabs, name='edges-slab-writer', daemon=True)
+        writer.start()
+        nbytes = C.c_int64()
+        total = 0
+        try:
+            for lo in range(0, n, chunk):
+                m = min(chunk, n - lo)
+                _cabi.check(_cabi.lib.b3c_edges_text(ws.data_ptr(), ws.numel(), u.data_ptr() + 4 * lo,
+                                                     v.data_ptr() + 4 * lo, w.data_ptr() + 8 * lo, m, sep_byte,
+                                                     int(float_style), text.data_ptr(), cap, C.byref(nbytes),
+                                                     C.c_void_p(stream.cuda_stream)))
+                k = free.get()
+                if k is None:
+                    break
+                nb = int(nbytes.value)
+                slabs[k][:nb].copy_(text[:nb], non_blocking=True)
+                stream.synchronize()
+                ready.put((k, nb))
+                total += nb
+        finally:
+            ready.put(None)
+            writer.join()
+        if failed:
+            raise failed[0]
+    return total

@@ -86,8 +86,14 @@ def write_edges(u, v, w, parent_dir, base_name='cm_graph', sep=' ', py2_str=Fals
     The file nx.write_edgelist(g, path, data=['weight'], delimiter=' ') produces (cluster.py:139-151):
     one 'u v weight' line per undirected edge.  networkx prints the weight with str(): repr(float) on
     Python 3 (the default here); `py2_str=True` gives what the Python 2.7 the reference pins prints
-    ('%.12g', '.0' appended to integer-looking values).  Written by the native writer of libbin3c_io.so
-    (include/bin3c_io.h: b3c_edges_write_fmt), formatted on a pool of threads.
+    ('%.12g', '.0' appended to integer-looking values).  Host arrays are written by the native writer of
+    libbin3c_io.so (include/bin3c_io.h: b3c_edges_write_fmt), formatted on a pool of threads.  u, v and w may also
+    be CUDA tensors, which are formatted on their device and leave it as text (bam_io.write_edges):
+
+        u, v, w, scl = to_edges(cm, norm=True, bisto=True, scale=True, device=True)
+        write_edges(u, v, w, out_dir, py2_str=True)
+
+    Either way the file is the same byte for byte.  Returns the path of the file.
     """
     from . import bam_io
     edge_file = os.path.join(parent_dir, '{}.edges'.format(base_name))

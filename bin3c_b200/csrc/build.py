@@ -11,8 +11,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.dirname(HERE)
 LIB = os.path.join(PKG, 'libbin3c_b200.so')
-SOURCES = ['core.cu', 'accum.cu', 'rowops.cu', 'kr.cu', 'synth.cu', 'bamdec.cu', 'sites.cu']
-HEADERS = ['common.cuh', 'inflate.cuh', 'sites.cuh', os.path.join('..', '..', 'include', 'bin3c_b200.h')]
+SOURCES = ['core.cu', 'accum.cu', 'rowops.cu', 'kr.cu', 'synth.cu', 'bamdec.cu', 'sites.cu', 'edgefmt.cu']
+HEADERS = ['common.cuh', 'inflate.cuh', 'sites.cuh', 'edgefmt.cuh', 'edgefmt_pow5.h', os.path.join('..', '..', 'include', 'bin3c_b200.h')]
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '-Xcompiler', '-fPIC', '--shared']
 

@@ -498,6 +498,26 @@ int b3c_sites_slab(void *d_ws, const uint8_t *d_bytes, int64_t n_bytes, int64_t 
 int b3c_sites_finish(void *d_ws, int64_t *d_seqs, int64_t *d_out, int64_t out_rows, int64_t *h_result,
                      void *stream);
 
+/* ------------------------------------------------------------------------------------
+ * The cm_graph.edges text of device edge arrays (bin3c_b200/csrc/edgefmt.cu, edgefmt.cuh): one line
+ * "u<sep>v<sep>weight\n" per edge, byte for byte what b3c_edges_write_fmt (include/bin3c_io.h) writes for
+ * the same host arrays.  float_style is B3C_FLOAT_REPR or B3C_FLOAT_STR12 of include/bin3c_io.h; sep is
+ * any byte (0..255).  A line takes at most B3C_EDGES_MAX_LINE_BYTES bytes (two 11-byte ids, two
+ * separators, the 24-byte "-d.dddddddddddddddde-308" and the newline).
+ *
+ *   workspace_bytes  scratch for calls of up to max_edges edges
+ *   text       d_u, d_v (int32) and d_w (float64) hold n_edges edges (device; may be NULL when
+ *              n_edges == 0); the text goes to d_text[0 .. *h_bytes) (device, any alignment: the
+ *              kernel stores 16-byte words only at 16-byte aligned addresses, and no byte outside
+ *              that range is written), text_capacity >= B3C_EDGES_MAX_LINE_BYTES * n_edges.
+ *              Synchronises the stream once.
+ * ------------------------------------------------------------------------------------ */
+#define B3C_EDGES_MAX_LINE_BYTES 49
+int64_t b3c_edges_text_workspace_bytes(int64_t max_edges);
+int b3c_edges_text(void *d_ws, int64_t ws_bytes, const int32_t *d_u, const int32_t *d_v, const double *d_w,
+                   int64_t n_edges, int32_t sep, int32_t float_style, uint8_t *d_text, int64_t text_capacity,
+                   int64_t *h_bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
