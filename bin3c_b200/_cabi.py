@@ -73,6 +73,7 @@ SIGNATURES = {
     'b3c_asymmetry_count': (C.c_int, [_i32, _p, _p, _p, _f64, _p, _pi64, _p]),
     'b3c_spmv': (C.c_int, [_i32, _i64, _p, _p, _p, _p, _p, _p, _i64, _i32, _p]),
     'b3c_set_option': (C.c_int, [_i32, _i64]),
+    'b3c_accum_plan': (C.c_int, [_i64, _i32, _i32, _pi64]),
     'b3c_peer_alloc': (C.c_int, [_i64, C.POINTER(C.c_void_p), C.c_char_p]),
     'b3c_peer_open': (C.c_int, [C.c_char_p, C.POINTER(C.c_void_p)]),
     'b3c_peer_close': (C.c_int, [_p]),

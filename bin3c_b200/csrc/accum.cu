@@ -684,6 +684,12 @@ __global__ void __launch_bounds__(RS_THREADS) k_rs_scatter(const uint64_t *__res
 // the lighter 256-bin kernels run.
 static int radix_passes(int bits) { return bits <= 0 ? 0 : (bits + RS_BITS - 1) / RS_BITS; }
 
+// bits per digit of radix_sort over `bits` bits (the last pass may take fewer); above 8 the 512-bin kernels run
+static int radix_digit(int bits) {
+    const int passes = radix_passes(bits);
+    return passes > 0 ? (bits + passes - 1) / passes : 0;
+}
+
 // which buffer (0 = a, 1 = b) holds the result of radix_sort over these bits: the parity of the pass count
 static int radix_where(int bit_lo, int bit_hi) { return radix_passes(bit_hi - bit_lo) & 1; }
 
@@ -702,7 +708,7 @@ static int radix_sort(uint64_t *a, uint64_t *b, const unsigned long long *d_n, i
                       uint32_t *d_hist, cudaStream_t s, int *where) {
     const int bits = bit_hi - bit_lo, passes = radix_passes(bits);
     const bool wide = passes > 0 && passes * 8 < bits;           // 8-bit digits would need another pass
-    const int digit = passes > 0 ? (bits + passes - 1) / passes : 0;
+    const int digit = radix_digit(bits);
     int cur = 0;
     for (int shift = bit_lo; shift < bit_hi; shift += digit) {
         const int w = (bit_hi - shift) < digit ? (bit_hi - shift) : digit;
@@ -1382,6 +1388,23 @@ int64_t b3c_accum_workspace_bytes(int64_t pair_capacity, int32_t n_seq, int32_t 
     AccumState st;
     plan(st, pair_capacity, n_seq, n_refs);
     return st.total;
+}
+
+int b3c_accum_plan(int64_t pair_capacity, int32_t n_seq, int32_t n_refs, int64_t *h_out) {
+    B3C_REQUIRE(h_out != nullptr && pair_capacity >= 0 && n_seq > 0 && n_refs > 0, "bad arguments");
+    AccumState st;
+    plan(st, pair_capacity, n_seq, n_refs);
+    h_out[0] = st.b;
+    h_out[1] = st.smem_diag ? 1 : 0;
+    h_out[2] = st.smem_rank;
+    h_out[3] = st.cls_cap_w;
+    h_out[4] = st.cls_diag_k;
+    h_out[5] = radix_passes(2 * st.b);              // key sort, bits [0, 2b)
+    h_out[6] = radix_digit(2 * st.b);
+    h_out[7] = radix_passes(st.b);                  // composite sort, its b column bits
+    h_out[8] = radix_digit(st.b);
+    h_out[9] = comp_cbits(st.b);
+    return B3C_OK;
 }
 
 int b3c_accum_begin(void *d_ws, int64_t ws_bytes, int64_t pair_capacity, int32_t n_seq,

@@ -207,6 +207,12 @@ int b3c_site_norm_f64(int32_t n_local, int32_t row_lo, const int64_t *d_indptr,
 enum { B3C_OPT_KR_SLAB_WIDTH = 1, B3C_OPT_KR_MAX_SLABS = 2, B3C_OPT_KR_FLAGS = 3, B3C_OPT_PEER_TIMEOUT_MS = 4,
        B3C_OPT_KR_COUNT_STREAM = 5, B3C_OPT_USE_GRAPHS = 6 };
 int b3c_set_option(int32_t key, int64_t value);
+/* b3c_accum_plan: the code paths an accumulator of these sizes takes (host-only, no CUDA call), so tests can
+ * assert the branch they were written for.  h_out[10] = key bits b per index, shared-memory diagonal (0/1),
+ * rank-table mode of the classify kernel (0 gather, 1 pair table, 2 packed table, 3 two-level table), staging
+ * keys per warp, contigs of the partial shared-memory diagonal, passes and digit bits of the key sort
+ * (bits [0, 2b)), passes and digit bits of the mirror composite's sort, count bits of the composite. */
+int b3c_accum_plan(int64_t pair_capacity, int32_t n_seq, int32_t n_refs, int64_t *h_out);
 
 int64_t b3c_kr_workspace_bytes(int32_t n, int64_t nnz);
 int b3c_kr_run(int32_t n, int64_t nnz, const int64_t *d_indptr, const int32_t *d_indices,
