@@ -11,7 +11,8 @@
 //                  counted in a shared-memory histogram (most Hi-C pairs are intra-contig),
 //                  off-diagonal pairs become keys (i << b | j), staged in shared memory and
 //                  appended to the key buffer with one global atomic per 4096-record tile.
-//   k_rs_*         LSD radix sort of the keys, 8-bit digits, only the 2b significant bits.
+//   k_rs_*         LSD radix sort of the keys, only the 2b significant bits, digits of up to 9 bits; the
+//                  scatter ranks each warp row through shared-memory peer masks (one atomicOr per key).
 //   k_rle_*        run-length reduce of the sorted keys -> unique (i,j) + exact counts.
 //   k_emit_*       upper and lower halves + diagonal scattered into canonical CSR; the lower
 //                  half's order comes from a stable sort of (j, e) on j's bits alone.
@@ -34,6 +35,10 @@ constexpr int SMEM_MAX = 232448;                 // 227 KB opt-in limit per CTA 
 constexpr int RS_THREADS = 512;
 constexpr int RS_KPT = 8;
 constexpr int RS_TILE = RS_THREADS * RS_KPT;
+// keys per thread of the radix passes: an 8192-key tile writes each 9-bit digit's keys out as a run of ~16 keys
+// (128 B), which measured faster than 4096-key tiles at two CTAs per SM and 16384-key tiles
+constexpr int RS_SORT_KPT = 16;
+constexpr int RS_SORT_TILE = RS_THREADS * RS_SORT_KPT;
 constexpr int RS_WARPS = RS_THREADS / 32;
 constexpr int RS_BITS = 9;                       // widest digit (k_rs_*<9>); k_rs_*<8> where it needs no more passes
 constexpr int RS_BINS = 1 << RS_BITS;            // sizes the histogram buffers
@@ -520,13 +525,14 @@ __global__ void k_accum_guard(unsigned long long *__restrict__ ctr, int64_t cap)
 }
 
 // ---- LSD radix sort --------------------------------------------------------------------
-__device__ __forceinline__ void rs_segment(int64_t n, int64_t *lo, int64_t *hi, int64_t *t0, int64_t *t1) {
-    const int64_t n_tiles = (n + RS_TILE - 1) / RS_TILE;
+__device__ __forceinline__ void rs_segment(int64_t n, int64_t *lo, int64_t *hi, int64_t *t0, int64_t *t1,
+                                           int tile_keys = RS_TILE) {
+    const int64_t n_tiles = (n + tile_keys - 1) / tile_keys;
     const int64_t tpb = (n_tiles + gridDim.x - 1) / gridDim.x;
     *t0 = min((int64_t)blockIdx.x * tpb, n_tiles);
     *t1 = min(*t0 + tpb, n_tiles);
-    *lo = *t0 * RS_TILE;
-    *hi = min(n, *t1 * RS_TILE);
+    *lo = *t0 * tile_keys;
+    *hi = min(n, *t1 * tile_keys);
 }
 
 template <int BITS>
@@ -538,7 +544,7 @@ __global__ void __launch_bounds__(RS_THREADS) k_rs_hist(const uint64_t *__restri
     for (int i = threadIdx.x; i < RS_BINS; i += RS_THREADS) s_h[i] = 0;
     __syncthreads();
     int64_t lo, hi, t0, t1;
-    rs_segment((int64_t)*d_n, &lo, &hi, &t0, &t1);
+    rs_segment((int64_t)*d_n, &lo, &hi, &t0, &t1, RS_SORT_TILE);
     for (int64_t i = lo + threadIdx.x; i < hi; i += RS_THREADS)
         atomicAdd(&s_h[(unsigned)(keys[i] >> shift) & mask], 1u);
     __syncthreads();
@@ -565,27 +571,38 @@ __global__ void __launch_bounds__(256) k_rs_scan_digit(uint32_t *__restrict__ hi
     if (threadIdx.x == 0) totals[blockIdx.x] = tot;
 }
 
+// Tile scatter: each warp ranks its 16 rows of 32 keys stably by digit.  The lanes of a row that share a digit find
+// each other through the warp's table of (peer mask, running count) pairs: every lane ORs its bit into the mask word of
+// its digit, reads the pair back, takes count + (peers below it) as its rank and leaves (0, count + peers) behind.  The
+// OR is order-free, so the rank is deterministic; per row that is one shared atomic, one 64-bit load and one 64-bit
+// store (match.any is a slow MIO operation on this part).  The digit pass then turns the per-warp counts into tile
+// offsets in place, the tile is staged in digit order and written out in runs.  The next tile's loads are issued as
+// soon as this tile's keys are staged, so they are in flight during the write-out.
 template <int BITS>
-__global__ void __launch_bounds__(RS_THREADS) k_rs_scatter(const uint64_t *__restrict__ in,
+__host__ __device__ constexpr int rs_scatter_smem() {
+    return RS_WARPS * (1 << BITS) * 8 + RS_SORT_TILE * 8;        // (mask, count) tables | staged keys
+}
+
+template <int BITS>
+__global__ void __launch_bounds__(RS_THREADS, 1) k_rs_scatter(const uint64_t *__restrict__ in,
                                                            uint64_t *__restrict__ out,
                                                            const unsigned long long *__restrict__ d_n, int shift,
                                                            unsigned mask, const uint32_t *__restrict__ offs,
                                                            const uint32_t *__restrict__ totals) {
-    constexpr int RS_BITS = BITS, RS_BINS = 1 << BITS;
+    constexpr int RS_BINS = 1 << BITS;
     static_assert(RS_BINS <= RS_THREADS, "one thread per digit");
-    __shared__ uint32_t s_wcnt[RS_WARPS][RS_BINS + 1];
     __shared__ uint32_t s_off[RS_BINS];
-    __shared__ uint32_t s_tot[RS_BINS];
-    __shared__ uint32_t s_bin[RS_BINS];
-    __shared__ uint32_t s_dst[RS_BINS];         // s_off - s_bin of the current tile: out index = s_dst[d] + q
+    __shared__ uint32_t s_dst[RS_BINS];         // out index of the tile's key q with digit d = s_dst[d] + q
     __shared__ uint32_t s_scan[33];
     extern __shared__ __align__(16) unsigned char rs_dyn[];
-    uint64_t *s_keys = reinterpret_cast<uint64_t *>(rs_dyn);     // RS_TILE keys (32 KB, dynamic)
+    uint2 *s_mc = reinterpret_cast<uint2 *>(rs_dyn);                          // [RS_WARPS][RS_BINS] (mask, count)
+    uint64_t *s_keys = reinterpret_cast<uint64_t *>(rs_dyn + RS_WARPS * RS_BINS * 8);   // RS_SORT_TILE staged keys
 
     const int64_t n = (int64_t)*d_n;
     int64_t lo, hi, t0, t1;
-    rs_segment(n, &lo, &hi, &t0, &t1);
+    rs_segment(n, &lo, &hi, &t0, &t1, RS_SORT_TILE);
     const unsigned lane = lane_id(), warp = threadIdx.x >> 5, lt = lanemask_lt();
+    uint2 *w_mc = s_mc + warp * RS_BINS;
     {
         // digit base = exclusive scan of the digit totals; plus this block's offset inside the digit
         const uint32_t v = (threadIdx.x < RS_BINS) ? totals[threadIdx.x] : 0u;
@@ -593,88 +610,73 @@ __global__ void __launch_bounds__(RS_THREADS) k_rs_scatter(const uint64_t *__res
         const uint32_t ex = block_scan_excl<uint32_t>(v, s_scan, &tot);
         if (threadIdx.x < RS_BINS) s_off[threadIdx.x] = ex + offs[(int64_t)threadIdx.x * gridDim.x + blockIdx.x];
     }
+    for (int i = lane; i < RS_BINS / 2; i += 32) reinterpret_cast<uint4 *>(w_mc)[i] = make_uint4(0u, 0u, 0u, 0u);
+    uint64_t key[RS_SORT_KPT];
+    const int kbase = warp * (32 * RS_SORT_KPT) + lane;                   // warp-striped: order == index order
+    auto load_tile = [&](int64_t tile) {
+        const int64_t base = tile * RS_SORT_TILE;
+        const int cnt = (int)min((int64_t)RS_SORT_TILE, n - base);
+#pragma unroll
+        for (int k = 0; k < RS_SORT_KPT; ++k) key[k] = (kbase + k * 32 < cnt) ? in[base + kbase + k * 32] : 0ull;
+    };
+    if (t0 < t1) load_tile(t0);
     __syncthreads();
 
     for (int64_t tile = t0; tile < t1; ++tile) {
-        const int64_t base = tile * RS_TILE;
-        const int cnt = (int)min((int64_t)RS_TILE, n - base);
-        for (int i = threadIdx.x; i < RS_WARPS * (RS_BINS + 1); i += RS_THREADS) (&s_wcnt[0][0])[i] = 0;
-        uint64_t key[RS_KPT];
-        uint32_t dg[RS_KPT], rk[RS_KPT];
+        const int cnt = (int)min((int64_t)RS_SORT_TILE, n - tile * RS_SORT_TILE);
+        uint32_t rk[RS_SORT_KPT];
 #pragma unroll
-        for (int k = 0; k < RS_KPT; ++k) {
-            const int idx = warp * (32 * RS_KPT) + k * 32 + lane;     // warp-striped: order == index order
-            const bool valid = idx < cnt;
-            key[k] = valid ? in[base + idx] : 0ull;
-            dg[k] = valid ? ((unsigned)(key[k] >> shift) & mask) : (unsigned)RS_BINS;
+        for (int k = 0; k < RS_SORT_KPT; ++k) {
+            const bool valid = kbase + k * 32 < cnt;
+            uint2 *p = w_mc + ((unsigned)(key[k] >> shift) & mask);
+            if (valid) atomicOr(&p->x, 1u << lane);
+            __syncwarp();
+            uint2 mc = make_uint2(0u, 0u);
+            if (valid) mc = *p;
+            __syncwarp();
+            rk[k] = mc.y + __popc(mc.x & lt);
+            if (valid) *p = make_uint2(0u, mc.y + __popc(mc.x));
+            __syncwarp();                          // row k's counts are in place before row k + 1's masks
         }
         __syncthreads();
-        // stable rank inside the warp, one item row at a time.  The peer masks do not depend on the counters, so
-        // they are all taken first; then the leader of every match group bumps the warp's digit counter with ONE
-        // shared-memory atomic that returns the count of the earlier rows (the rows' atomics are issued back to
-        // back: nothing waits for a value until the shuffles below), and the group reads it from the leader.
-        unsigned mm[RS_KPT];
-#pragma unroll
-        for (int k = 0; k < RS_KPT; ++k) {
-            // lanes holding the same digit: one ballot per digit bit (match.any is a slow MIO operation here --
-            // it was 24 % of this kernel's stall samples); invalid lanes (digit RS_BINS) form their own group
-            const bool valid = dg[k] < (unsigned)RS_BINS;
-            unsigned m = __ballot_sync(kFullMask, valid);
-            if (!valid) m = ~m;
-#pragma unroll
-            for (int b = 0; b < RS_BITS; ++b) {
-                const bool bit = (dg[k] >> b) & 1u;
-                const unsigned bal = __ballot_sync(kFullMask, bit);
-                m &= bit ? bal : ~bal;
-            }
-            mm[k] = m;
-        }
-#pragma unroll
-        for (int k = 0; k < RS_KPT; ++k) {
-            rk[k] = 0;
-            if ((int)lane == __ffs(mm[k]) - 1) rk[k] = atomicAdd(&s_wcnt[warp][dg[k]], (uint32_t)__popc(mm[k]));
-            __syncwarp();                          // row k's additions are ordered before row k + 1's
-        }
-#pragma unroll
-        for (int k = 0; k < RS_KPT; ++k)
-            rk[k] = __shfl_sync(kFullMask, rk[k], __ffs(mm[k]) - 1) + __popc(mm[k] & lt);
-        __syncthreads();
-        // per digit: exclusive scan over warps, tile total
-        if (threadIdx.x < RS_BINS) {
-            uint32_t run = 0;
-#pragma unroll
-            for (int w = 0; w < RS_WARPS; ++w) {
-                const uint32_t c = s_wcnt[w][threadIdx.x];
-                s_wcnt[w][threadIdx.x] = run;
-                run += c;
-            }
-            s_tot[threadIdx.x] = run;
-        }
-        __syncthreads();
+        // per digit: tile total, exclusive scan over digits, then each warp's count becomes its first tile slot
         {
-            const uint32_t v = (threadIdx.x < RS_BINS) ? s_tot[threadIdx.x] : 0u;
+            const int d = threadIdx.x;
+            uint32_t v = 0;
+            if (d < RS_BINS) {
+#pragma unroll
+                for (int w = 0; w < RS_WARPS; ++w) v += s_mc[w * RS_BINS + d].y;
+            }
             uint32_t tot;
-            const uint32_t ex = block_scan_excl<uint32_t>(v, s_scan, &tot);
-            if (threadIdx.x < RS_BINS) {
-                // digit d's keys of this tile go to out[s_off[d] ...]; thread d alone touches s_off[d], so it moves
-                // on to the next tile here (the write-out below reads s_dst): no barrier at the end of the tile
-                s_bin[threadIdx.x] = ex;
-                s_dst[threadIdx.x] = s_off[threadIdx.x] - ex;            // (mod 2^32, undone by + q below)
-                s_off[threadIdx.x] += v;
+            uint32_t run = block_scan_excl<uint32_t>(v, s_scan, &tot);
+            if (d < RS_BINS) {
+                // thread d alone touches s_off[d] / s_dst[d]; the write-out of the previous tile is behind the
+                // barriers of the scan
+                s_dst[d] = s_off[d] - run;                               // (mod 2^32, undone by + q below)
+                s_off[d] += v;
+#pragma unroll
+                for (int w = 0; w < RS_WARPS; ++w) {
+                    const uint32_t c = s_mc[w * RS_BINS + d].y;
+                    s_mc[w * RS_BINS + d].y = run;
+                    run += c;
+                }
             }
         }
         __syncthreads();
 #pragma unroll
-        for (int k = 0; k < RS_KPT; ++k)
-            if (dg[k] < (unsigned)RS_BINS) s_keys[s_bin[dg[k]] + s_wcnt[warp][dg[k]] + rk[k]] = key[k];
+        for (int k = 0; k < RS_SORT_KPT; ++k)
+            if (kbase + k * 32 < cnt) s_keys[w_mc[(unsigned)(key[k] >> shift) & mask].y + rk[k]] = key[k];
+        __syncwarp();
+        // this warp's table is read by no one else until the next tile's digit pass: zero it for the next ranking
+        for (int i = lane; i < RS_BINS / 2; i += 32) reinterpret_cast<uint4 *>(w_mc)[i] = make_uint4(0u, 0u, 0u, 0u);
+        if (tile + 1 < t1) load_tile(tile + 1);
         __syncthreads();
         for (int q = threadIdx.x; q < cnt; q += RS_THREADS) {
             const uint64_t kk = s_keys[q];
             const unsigned d = (unsigned)(kk >> shift) & mask;
             out[(int64_t)(uint32_t)(s_dst[d] + (uint32_t)q)] = kk;
         }
-        // the next tile's first writes to s_wcnt / s_keys / s_tot / s_bin / s_dst all lie behind its own barriers;
-        // s_wcnt (zeroed at the top) was last read before the barrier above
+        // the next tile's first writes to s_keys and s_dst lie behind its own barriers
     }
 }
 
@@ -697,8 +699,8 @@ static int radix_where(int bit_lo, int bit_hi) { return radix_passes(bit_hi - bi
 static int radix_init() {
     static bool attr_done = false;
     if (!attr_done) {
-        B3C_CUDA(cudaFuncSetAttribute(k_rs_scatter<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, RS_TILE * 8));
-        B3C_CUDA(cudaFuncSetAttribute(k_rs_scatter<9>, cudaFuncAttributeMaxDynamicSharedMemorySize, RS_TILE * 8));
+        B3C_CUDA(cudaFuncSetAttribute(k_rs_scatter<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, rs_scatter_smem<8>()));
+        B3C_CUDA(cudaFuncSetAttribute(k_rs_scatter<9>, cudaFuncAttributeMaxDynamicSharedMemorySize, rs_scatter_smem<9>()));
         attr_done = true;
     }
     return B3C_OK;
@@ -722,8 +724,8 @@ static int radix_sort(uint64_t *a, uint64_t *b, const unsigned long long *d_n, i
         B3C_LAUNCH_CHECK();
         k_rs_scan_digit<<<bins, 256, 0, s>>>(d_hist, RS_BLOCKS, d_totals);
         B3C_LAUNCH_CHECK();
-        if (wide) k_rs_scatter<9><<<RS_BLOCKS, RS_THREADS, RS_TILE * 8, s>>>(src, dst, d_n, shift, mask, d_hist, d_totals);
-        else k_rs_scatter<8><<<RS_BLOCKS, RS_THREADS, RS_TILE * 8, s>>>(src, dst, d_n, shift, mask, d_hist, d_totals);
+        if (wide) k_rs_scatter<9><<<RS_BLOCKS, RS_THREADS, rs_scatter_smem<9>(), s>>>(src, dst, d_n, shift, mask, d_hist, d_totals);
+        else k_rs_scatter<8><<<RS_BLOCKS, RS_THREADS, rs_scatter_smem<8>(), s>>>(src, dst, d_n, shift, mask, d_hist, d_totals);
         B3C_LAUNCH_CHECK();
         cur ^= 1;
     }
