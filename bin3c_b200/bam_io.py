@@ -279,15 +279,14 @@ def pair_records_from_bam(path, sites=None, min_mapq=60, strong=None, min_insert
 
 def _pair_records_on_device(path, sites, min_mapq, strong, min_insert, min_len, slab_bytes, slab_blocks):
     """
-    pair_records_from_bam(device=True).  One host thread reads the file into two pinned slabs and lists each slab's
-    BGZF blocks (b3c_bgzf_scan) while the device decodes the previous slab (include/bin3c_b200.h: b3c_bamdec_*); each
-    slab goes to the device with one asynchronous copy, and the record tensor grows as slabs finish.
+    pair_records_from_bam(device=True).  A read-ahead slab ring reads the file into two pinned slabs and lists each
+    slab's BGZF blocks (b3c_bgzf_scan) while the device decodes the previous slab (include/bin3c_b200.h:
+    b3c_bamdec_*); each slab goes to the device with one asynchronous copy, and the record tensor grows as slabs finish.
     """
-    import queue
-    import threading
     import torch
-    from . import _cabi
+    from . import _cabi, slab_ring
     from .contact_map import PairRecords
+    from .device import grown
     if not torch.cuda.is_available():
         raise RuntimeError('pair_records_from_bam(device=True) needs a CUDA device; the host reader is device=False')
     with BamPairReader(path, threads=1) as bam:                 # header, sort order, reference table
@@ -315,60 +314,36 @@ def _pair_records_on_device(path, sites, min_mapq, strong, min_insert, min_len, 
                                            n_refs, data_offset, stream))
 
     pinned = [torch.empty(cap, dtype=torch.uint8, pin_memory=True) for _ in range(2)]
-    free, ready = queue.Queue(), queue.Queue()
-    for k in range(2):
-        free.put(k)
+    left, eof = np.empty(0, dtype=np.uint8), False
 
-    def read_slabs():
-        try:
-            left = np.empty(0, dtype=np.uint8)
-            eof = False
-            with open(path, 'rb') as f:
-                while True:
-                    k = free.get()
-                    if k is None:
-                        return
-                    a = pinned[k].numpy()
-                    n = len(left)
-                    a[:n] = left
-                    while n < cap and not eof:
-                        m = f.readinto(memoryview(a)[n:cap])
-                        eof = not m
-                        n += m or 0
-                    offs = np.empty(max_blocks, dtype=np.int64)
-                    bsz = np.empty(max_blocks, dtype=np.int32)
-                    isz = np.empty(max_blocks, dtype=np.int32)
-                    used = np.zeros(1, dtype=np.int64)
-                    nb = lib.b3c_bgzf_scan(a.ctypes.data, n, 1 if eof else 0, offs.ctypes.data, bsz.ctypes.data,
-                                           isz.ctypes.data, max_blocks, used.ctypes.data)
-                    if nb < 0:
-                        ready.put(('error', nb, '{}: {}'.format(path, last_error())))
-                        return
-                    c = int(used[0])
-                    left = a[c:n].copy()
-                    last = eof and c == n
-                    ready.put((k, int(nb), c, offs[:nb], bsz[:nb], isz[:nb], last))
-                    if last:
-                        return
-        except BaseException as e:                              # handed to the decoding thread
-            ready.put(('error', None, e))
+    def fill(a):                                                # the ring's thread: the carried bytes, then the file
+        nonlocal left, eof
+        n = len(left)
+        a[:n] = left
+        while n < cap and not eof:
+            m = f.readinto(memoryview(a)[n:cap])
+            eof = not m
+            n += m or 0
+        offs = np.empty(max_blocks, dtype=np.int64)
+        bsz = np.empty(max_blocks, dtype=np.int32)
+        isz = np.empty(max_blocks, dtype=np.int32)
+        used = np.zeros(1, dtype=np.int64)
+        nb = lib.b3c_bgzf_scan(a.ctypes.data, n, 1 if eof else 0, offs.ctypes.data, bsz.ctypes.data,
+                               isz.ctypes.data, max_blocks, used.ctypes.data)
+        if nb < 0:
+            raise ValueError('{}: {}'.format(path, last_error()))  # the reader's status for a bad BGZF block
+        c = int(used[0])
+        left = a[c:n].copy()
+        return int(nb), c, offs[:nb], bsz[:nb], isz[:nb], eof and c == n
 
-    reader = threading.Thread(target=read_slabs, name='bam-slab-reader', daemon=True)
-    reader.start()
-    d_comp = torch.empty(cap, dtype=torch.uint8, device=dev)
-    u_bufs = [None, None]
-    out = torch.empty(1 << 20, dtype=torch.uint64, device=dev)
-    n_out, stream_off, next_rec = 0, 0, data_offset
-    prev_u, prev_u0, repaired, n_slabs = None, 0, 0, 0
-    res = (C.c_int64 * 4)()
-    try:
-        while True:
-            item = ready.get()
-            if item[0] == 'error':
-                if item[1] is None:
-                    raise item[2]
-                raise ValueError(item[2])                       # the reader's status for a bad BGZF block
-            k, nb, c, offs, bsz, isz, last = item
+    with open(path, 'rb') as f, slab_ring.SlabRing([p.numpy() for p in pinned], fill=fill) as ring:
+        d_comp = torch.empty(cap, dtype=torch.uint8, device=dev)
+        u_bufs = [None, None]
+        out = torch.empty(1 << 20, dtype=torch.uint64, device=dev)
+        n_out, stream_off, next_rec = 0, 0, data_offset
+        prev_u, prev_u0, repaired, n_slabs = None, 0, 0, 0
+        res = (C.c_int64 * 4)()
+        for k, (nb, c, offs, bsz, isz, last) in ring:
             tbl = np.empty((nb, 3), dtype=np.int64)
             tbl[:, 0] = offs
             tbl[:, 1] = bsz.astype(np.int64) | (isz.astype(np.int64) << 32)
@@ -385,9 +360,7 @@ def _pair_records_on_device(path, sites, min_mapq, strong, min_insert, min_len, 
             d_carry = prev_u.data_ptr() + (next_rec - prev_u0) if carry else None
             bound = need // 72 + 2
             if out.numel() - n_out < bound:
-                grown = torch.empty(max(2 * out.numel(), n_out + bound), dtype=torch.uint64, device=dev)
-                grown[:n_out].copy_(out[:n_out])
-                out = grown
+                out = grown(out, max(2 * out.numel(), n_out + bound), n_out)
             if c:
                 d_comp[:c].copy_(pinned[k][:c], non_blocking=True)
             d_tbl = torch.from_numpy(tbl.reshape(-1)).pin_memory().to(dev, non_blocking=True) if nb else None
@@ -395,7 +368,7 @@ def _pair_records_on_device(path, sites, min_mapq, strong, min_insert, min_len, 
                                            stream_off, u_bytes, d_carry, carry, u.data_ptr(), u.numel(),
                                            1 if last else 0, out.data_ptr() + 8 * n_out, out.numel() - n_out, res,
                                            stream)
-            free.put(k)                                         # the slab call synchronised: the pinned slab is free
+            ring.release(k)                                     # the slab call synchronised: the pinned slab is free
             if rc == _cabi.B3C_ERR_FORMAT:
                 raise ValueError('{}: {}'.format(path, _cabi.last_error()))
             _cabi.check(rc)
@@ -405,11 +378,6 @@ def _pair_records_on_device(path, sites, min_mapq, strong, min_insert, min_len, 
             repaired += int(res[2])
             stream_off += u_bytes
             n_slabs += 1
-            if last:
-                break
-    finally:
-        free.put(None)
-        reader.join()
     st = np.zeros(8, dtype=np.int64)
     _cabi.check(_cabi.lib.b3c_bamdec_stats(ws.data_ptr(), st.ctypes.data_as(C.POINTER(C.c_int64)), 8, stream))
     stats = dict(zip(STAT_NAMES, st.tolist() + [0]))
@@ -514,13 +482,11 @@ DEFAULT_EDGE_CHUNK = 1 << 21      # edges per device formatting call (text buffe
 def _write_edges_on_device(u, v, w, path, sep=' ', float_style=FLOAT_REPR, chunk_edges=DEFAULT_EDGE_CHUNK):
     """
     write_edges for CUDA tensors.  The device formats chunk_edges edges at a time into a text buffer
-    (include/bin3c_b200.h: b3c_edges_text); each chunk's text is copied into one of two pinned host slabs, and one
-    writer thread writes slab k to the file while the device formats chunk k + 1.  Returns the bytes written.
+    (include/bin3c_b200.h: b3c_edges_text); each chunk's text is copied into one of two pinned host slabs, and a
+    write-behind slab ring writes slab k to the file while the device formats chunk k + 1.  Returns the bytes written.
     """
-    import queue
-    import threading
     import torch
-    from . import _cabi
+    from . import _cabi, slab_ring
     assert len(u) == len(v) == len(w)
     assert isinstance(sep, str) and len(sep) == 1, 'single-character separator'
     sep_byte = sep.encode('ascii')[0]
@@ -541,46 +507,19 @@ def _write_edges_on_device(u, v, w, path, sep=' ', float_style=FLOAT_REPR, chunk
         ws = torch.empty(int(_cabi.lib.b3c_edges_text_workspace_bytes(chunk)), dtype=torch.uint8, device=dev)
         text = torch.empty(cap, dtype=torch.uint8, device=dev)
         slabs = [torch.empty(cap, dtype=torch.uint8, pin_memory=True) for _ in range(2 if n > chunk else 1)]
-        free, ready = queue.Queue(), queue.Queue()
-        for k in range(len(slabs)):
-            free.put(k)
-        failed = []
-
-        def write_slabs():
-            try:
-                while True:
-                    item = ready.get()
-                    if item is None:
-                        return
-                    k, nb = item
-                    f.write(memoryview(slabs[k].numpy())[:nb])
-                    free.put(k)
-            except BaseException as e:                          # handed to the formatting thread
-                failed.append(e)
-                free.put(None)
-
-        writer = threading.Thread(target=write_slabs, name='edges-slab-writer', daemon=True)
-        writer.start()
         nbytes = C.c_int64()
         total = 0
-        try:
+        with slab_ring.SlabRing([s.numpy() for s in slabs], drain=lambda a, nb: f.write(memoryview(a)[:nb])) as ring:
             for lo in range(0, n, chunk):
                 m = min(chunk, n - lo)
                 _cabi.check(_cabi.lib.b3c_edges_text(ws.data_ptr(), ws.numel(), u.data_ptr() + 4 * lo,
                                                      v.data_ptr() + 4 * lo, w.data_ptr() + 8 * lo, m, sep_byte,
                                                      int(float_style), text.data_ptr(), cap, C.byref(nbytes),
                                                      C.c_void_p(stream.cuda_stream)))
-                k = free.get()
-                if k is None:
-                    break
+                k = ring.acquire()
                 nb = int(nbytes.value)
                 slabs[k][:nb].copy_(text[:nb], non_blocking=True)
                 stream.synchronize()
-                ready.put((k, nb))
+                ring.release(k, nb)
                 total += nb
-        finally:
-            ready.put(None)
-            writer.join()
-        if failed:
-            raise failed[0]
     return total

@@ -98,6 +98,13 @@ class BufferPool(object):
         return t[:n]
 
 
+def grown(t, rows, keep):
+    """A larger buffer for a full one: a tensor like t with `rows` rows (dim 0), holding t's first `keep` rows."""
+    g = torch.empty((int(rows),) + tuple(t.shape[1:]), dtype=t.dtype, device=t.device)
+    g[:keep].copy_(t[:keep])
+    return g
+
+
 def _alloc(pool, name, n, dtype):
     return _empty(n, dtype) if pool is None else pool.get(name, n, dtype)
 

@@ -149,18 +149,17 @@ def site_table_from_rows(rows, names, min_len, tip_size):
 
 def _site_table_on_device(path, patterns, min_len, tip_size, slab_bytes, timing=None):
     """
-    fasta_site_table(device=True).  One host thread reads (and inflates) the file into two pinned slabs while the
-    device counts the previous one (include/bin3c_b200.h: b3c_sites_*); each slab crosses with one asynchronous copy
-    and one synchronisation.  The per-sequence table and the name arena stay on the device until the end.
+    fasta_site_table(device=True).  A read-ahead slab ring reads (and inflates) the file into two pinned slabs while
+    the device counts the previous one (include/bin3c_b200.h: b3c_sites_*); each slab crosses with one asynchronous
+    copy and one synchronisation.  The per-sequence table and the name arena stay on the device until the end.
     `timing`: a dict that receives the seconds spent reading / inflating, in slab calls, and waiting for the reader.
     """
     import ctypes as C
-    import queue
-    import threading
     import torch
     if not torch.cuda.is_available():
         raise RuntimeError('fasta_site_table(device=True) needs a CUDA device; the host counter is device=False')
-    from . import _cabi
+    from . import _cabi, slab_ring
+    from .device import grown
     masks, lengths, weights = patterns
     slab = max(1, min(int(slab_bytes), MAX_SLAB_BYTES))
     tip = int(tip_size) if tip_size else 0
@@ -172,47 +171,29 @@ def _site_table_on_device(path, patterns, min_len, tip_size, slab_bytes, timing=
     _cabi.check(_cabi.lib.b3c_sites_begin(ws.data_ptr(), nws, slab, masks.ctypes.data, lengths.ctypes.data,
                                           weights.ctypes.data, len(lengths), tip, stream))
     pinned = [torch.empty(slab, dtype=torch.uint8, pin_memory=True) for _ in range(2)]
-    free, ready = queue.Queue(), queue.Queue()
-    for k in range(2):
-        free.put(k)
     t = {'read_s': 0.0, 'slab_s': 0.0, 'wait_s': 0.0, 'slabs': 0, 'bytes': 0}
 
-    def read_slabs():
-        try:
-            gz = str(path).endswith('.gz')
-            with (gzip.open(path, 'rb') if gz else open(path, 'rb', buffering=0)) as f:
-                while True:
-                    k = free.get()
-                    if k is None:
-                        return
-                    view = memoryview(pinned[k].numpy())
-                    n, t0 = 0, time.perf_counter()
-                    while n < slab:
-                        m = f.readinto(view[n:])
-                        if not m:
-                            break
-                        n += m
-                    t['read_s'] += time.perf_counter() - t0
-                    ready.put((k, n))
-                    if n < slab:
-                        return
-        except BaseException as e:                              # handed to the counting thread
-            ready.put((None, e))
+    def fill(a):                                                # the ring's thread: a full slab, or up to the end
+        view = memoryview(a)
+        n, t0 = 0, time.perf_counter()
+        while n < slab:
+            m = f.readinto(view[n:])
+            if not m:
+                break
+            n += m
+        t['read_s'] += time.perf_counter() - t0
+        return n, n < slab
 
-    reader = threading.Thread(target=read_slabs, name='fasta-slab-reader', daemon=True)
-    reader.start()
-    d_buf = torch.empty(slab, dtype=torch.uint8, device=dev)
-    seq_cap, name_cap = 1 << 12, 1 << 16
-    seqs = torch.empty((seq_cap, 5), dtype=torch.int64, device=dev)
-    names = torch.empty(name_cap, dtype=torch.uint8, device=dev)
-    res = (C.c_int64 * 3)()
-    try:
-        while True:
-            t0 = time.perf_counter()
-            k, n = ready.get()
+    f = gzip.open(path, 'rb') if str(path).endswith('.gz') else open(path, 'rb', buffering=0)
+    with f, slab_ring.SlabRing([p.numpy() for p in pinned], fill=fill) as ring:
+        d_buf = torch.empty(slab, dtype=torch.uint8, device=dev)
+        seq_cap, name_cap = 1 << 12, 1 << 16
+        seqs = torch.empty((seq_cap, 5), dtype=torch.int64, device=dev)
+        names = torch.empty(name_cap, dtype=torch.uint8, device=dev)
+        res = (C.c_int64 * 3)()
+        t0 = time.perf_counter()
+        for k, (n, _) in ring:
             t['wait_s'] += time.perf_counter() - t0
-            if k is None:
-                raise n
             if n == 0:
                 break
             t0 = time.perf_counter()
@@ -224,15 +205,11 @@ def _site_table_on_device(path, patterns, min_len, tip_size, slab_bytes, timing=
                     break
                 if res[0] > seq_cap:                            # grow, keep what is written, count the slab again
                     seq_cap = max(2 * seq_cap, int(res[0]))
-                    grown = torch.empty((seq_cap, 5), dtype=torch.int64, device=dev)
-                    grown[:len(seqs)].copy_(seqs)
-                    seqs = grown
+                    seqs = grown(seqs, seq_cap, len(seqs))
                 if res[1] > name_cap:
                     name_cap = max(2 * name_cap, int(res[1]))
-                    grown = torch.empty(name_cap, dtype=torch.uint8, device=dev)
-                    grown[:len(names)].copy_(names)
-                    names = grown
-            free.put(k)                                         # the slab call synchronised: the pinned slab is free
+                    names = grown(names, name_cap, len(names))
+            ring.release(k)                                     # the slab call synchronised: the pinned slab is free
             t['slab_s'] += time.perf_counter() - t0
             t['slabs'] += 1
             t['bytes'] += n
@@ -240,11 +217,7 @@ def _site_table_on_device(path, patterns, min_len, tip_size, slab_bytes, timing=
                 raise ValueError('{}: {}; count this file with the host counter (device=False)'.format(
                     path, _cabi.last_error()))
             _cabi.check(rc)
-            if n < slab:
-                break
-    finally:
-        free.put(None)
-        reader.join()
+            t0 = time.perf_counter()
     n_seq = int(res[0])
     out = torch.empty((max(n_seq, 1), 5), dtype=torch.int64, device=dev)
     _cabi.check(_cabi.lib.b3c_sites_finish(ws.data_ptr(), seqs.data_ptr(), out.data_ptr(), n_seq, res, stream))
