@@ -1831,8 +1831,10 @@ __global__ void __launch_bounds__(1024) k_big_build(KRArgs A) {
     }
 }
 
-// ---- stand-alone kernels (microbench SpMV, host-driven phases) ------------------------------------
-template <bool SLAB>
+// ---- stand-alone kernels (microbench SpMV, host-driven phases, test hook) ----------------------------
+// The multiplied vector is A.u: u itself for an fp64 stream (b3c_spmv, the phase API), or the staged u / s or x / s
+// that b3c_kr_rowsum hands over in A.u for a counts stream (CNT 1 or 2, as k_kr_persistent).
+template <bool SLAB, int CNT>
 __global__ void __launch_bounds__(KR_THREADS, 1) k_spmv(KRArgs A) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem sm = carve_smem(smem_raw);
@@ -1840,7 +1842,30 @@ __global__ void __launch_bounds__(KR_THREADS, 1) k_spmv(KRArgs A) {
         if (threadIdx.x == 0) mbar_init(sm.mbar, 1);
         __syncthreads();
     }
-    phase_spmv<SLAB, 0>(A, A.u, sm);
+    phase_spmv<SLAB, CNT>(A, A.u, sm);
+}
+// b3c_kr_rowsum: v staged as the KR phases stage their operand (put_x, phase_dir_all): opnd = v and, counts form,
+// scaled = v * (1 / s) with the same rounding
+__global__ void __launch_bounds__(256) k_kr_stage(int32_t n, const double *__restrict__ v, const double *__restrict__ inv_s,
+                                                  double *__restrict__ opnd, double *__restrict__ scaled) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const double x = v[i];
+    opnd[i] = x;
+    if (scaled) scaled[i] = __dmul_rn(x, __ldg(inv_s + i));
+}
+// b3c_kr_rowsum: the row sums of the local rows as phase_resid reads them (boundary_fix, then rows_q), one CTA per
+// local chunk; q is indexed by local row
+__global__ void __launch_bounds__(KR_THREADS) k_kr_rowsum(KRArgs A, const double *opnd, double *__restrict__ q) {
+    const int c = A.row_lo / CHUNK + (int)blockIdx.x;
+    double qq[CHUNK_RPT];
+    boundary_fix(A, c);
+    rows_q(A, opnd, c, qq);
+#pragma unroll
+    for (int i = 0; i < CHUNK_RPT; ++i) {
+        const int64_t r = KR_ROW(c, i);
+        if (r < A.row_hi) q[r - A.row_lo] = qq[i];
+    }
 }
 // y[r] = (A u)[r] (b3c_spmv): one CTA per reduction chunk
 __global__ void __launch_bounds__(KR_THREADS) k_spmv_collect(KRArgs A, double *__restrict__ y) {
@@ -1951,7 +1976,10 @@ struct KRLayout {
     int64_t o_cnt, o_vp, o_ord, o_scan, o_slab_t0, o_sval, o_scol, o_sflag, o_seg0, o_seg_of, o_seg_row, o_big, o_cstart, total;
 };
 
-// `rows`: rows of the block the stream is built for (n for a whole matrix): the density rule counts the block's cells
+// `rows`: rows of the block the stream is built for (n for a whole matrix): the density rule counts the block's cells,
+// and those are laid out for its rows padded to whole reduction chunks (npad, so nv = S * npad).  Counting the padded
+// rows keeps a tail block of fewer than CHUNK rows in the form a CHUNK-row block with the same entries takes, which is
+// what b3c_krp_workspace_bytes sizes for.
 // `packed`: the stream will hold packed counts (b3c_kr_run*_counts with B3C_OPT_KR_COUNT_STREAM = 2)
 static KRLayout kr_layout(int32_t n, int64_t nnz, int32_t rows, bool packed = false) {
     KRLayout L;
@@ -1965,7 +1993,7 @@ static KRLayout kr_layout(int32_t n, int64_t nnz, int32_t rows, bool packed = fa
     // (the packed count stream moves 4 B per padded entry against the gather form's 8 B plus an L1 wavefront per entry:
     // measured on C4's row blocks at 6 entries per cell, 1.9 us per million entries against 3.9)
     const int dense = packed ? SLAB_DENSE_CELL_PACKED : SLAB_DENSE_CELL;
-    const bool dense_cells = s_max >= SLAB_S_MAX && s_need <= SLAB_S_CAP && nnz >= dense * (int64_t)rows * s_need;
+    const bool dense_cells = s_max >= SLAB_S_MAX && s_need <= SLAB_S_CAP && nnz >= dense * align_up(rows, CHUNK) * s_need;
     L.slab = (s_need <= s_max || dense_cells) ? 1 : 0;
     L.S = L.slab ? (int32_t)s_need : 1;
     L.W = L.slab ? (int32_t)align_up(ceil_div(n, L.S), 2) : n;
@@ -2105,7 +2133,9 @@ static int persistent_grid_of(int *grid_out) {
         B3C_CUDA(cudaFuncSetAttribute(k_kr_persistent<SLAB, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         B3C_CUDA(cudaFuncSetAttribute(k_kr_persistent<SLAB, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         if (SLAB) B3C_CUDA(cudaFuncSetAttribute(k_kr_persistent<true, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        B3C_CUDA(cudaFuncSetAttribute(k_spmv<SLAB>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        B3C_CUDA(cudaFuncSetAttribute(k_spmv<SLAB, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        B3C_CUDA(cudaFuncSetAttribute(k_spmv<SLAB, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        if (SLAB) B3C_CUDA(cudaFuncSetAttribute(k_spmv<true, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         B3C_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_kr_persistent<SLAB, 0>, KR_THREADS, smem));
         B3C_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_c, k_kr_persistent<SLAB, 1>, KR_THREADS, smem));
         if (per_sm < 1 || per_sm_c < 1) {
@@ -2223,9 +2253,16 @@ static int kr_prepare(KRArgs &A, const KRLayout &L, cudaStream_t s) {
     return A.slab ? kr_prepare_t<true>(A, L, s) : kr_prepare_t<false>(A, L, s);
 }
 
+// the stand-alone SpMV of the stream's form; A.u is the vector it multiplies (see k_spmv)
 static int launch_spmv(const KRArgs &A, cudaStream_t s) {
-    if (A.slab) k_spmv<true><<<A.n_bnd, KR_THREADS, SM_BYTES_SLAB, s>>>(A);
-    else k_spmv<false><<<A.n_bnd, KR_THREADS, SM_BYTES_GATHER, s>>>(A);
+    if (A.slab) {
+        if (A.cnt_stream == 2) k_spmv<true, 2><<<A.n_bnd, KR_THREADS, SM_BYTES_SLAB, s>>>(A);
+        else if (A.cnt_stream) k_spmv<true, 1><<<A.n_bnd, KR_THREADS, SM_BYTES_SLAB, s>>>(A);
+        else k_spmv<true, 0><<<A.n_bnd, KR_THREADS, SM_BYTES_SLAB, s>>>(A);
+    } else {
+        if (A.cnt_stream) k_spmv<false, 1><<<A.n_bnd, KR_THREADS, SM_BYTES_GATHER, s>>>(A);
+        else k_spmv<false, 0><<<A.n_bnd, KR_THREADS, SM_BYTES_GATHER, s>>>(A);
+    }
     B3C_LAUNCH_CHECK();
     return B3C_OK;
 }
@@ -2360,28 +2397,46 @@ static int kr_launch_collect(KRArgs &A, int32_t max_iter, double *d_x, int64_t *
     return B3C_OK;
 }
 
+// The stream form a counts matrix asks for under the current options (before the build's fall-back from 2 to 1)
+static int32_t kr_cnt_stream(bool counts, bool slab) {
+    const int cs = g_cnt_stream.load();
+    return (counts && cs) ? ((cs == 2 && slab) ? 2 : 1) : 0;
+}
+
+// The SpMV operand of rows [row_lo, row_hi) as every KR entry point builds it: layout (the density rule over the
+// block's rows), binding, the count-stream form, the control block, the stream with its side list and dfix.
+// kr_run_impl, kr_run_peer_impl and b3c_kr_rowsum all go through here, so what the test hook sums is the product's
+// operand.
+static int kr_operand(KRArgs &A, KRLayout &L, int32_t n, int32_t row_lo, int32_t row_hi, int64_t nnz,
+                      const int64_t *d_indptr, const int32_t *d_indices, const double *d_data, const uint32_t *d_counts,
+                      const int32_t *d_sites, double tol, double delta, double Delta, int32_t max_iter, void *d_ws,
+                      int64_t ws_bytes, cudaStream_t s) {
+    L = kr_layout(n, nnz, row_hi - row_lo, !d_data && d_counts && g_cnt_stream.load() == 2);
+    if (ws_bytes < L.total) {
+        set_error("KR workspace too small: %lld < %lld", (long long)ws_bytes, (long long)L.total);
+        return B3C_ERR_CAPACITY;
+    }
+    kr_bind(A, L, (char *)d_ws, n, row_lo, row_hi, nnz, d_indptr, d_indices, d_data);
+    A.cnt32 = d_data ? nullptr : d_counts;
+    A.sites = d_data ? nullptr : d_sites;
+    A.cnt_stream = kr_cnt_stream(A.cnt32 != nullptr, A.slab);
+    KRScalars S;
+    kr_scalars_init(S, tol, delta, Delta, max_iter);
+    B3C_CUDA(cudaMemcpyAsync(A.ctl, &S, sizeof(S), cudaMemcpyHostToDevice, s));
+    B3C_CUDA(cudaMemsetAsync(A.timers, 0, sizeof(KRTimers), s));
+    return kr_prepare(A, L, s);
+}
+
 static int kr_run_impl(int32_t n, int64_t nnz, const int64_t *d_indptr, const int32_t *d_indices, const double *d_data,
                        const uint32_t *d_counts, const int32_t *d_sites, double tol, double delta, double Delta,
                        int32_t max_iter, double *d_x, void *d_ws, int64_t ws_bytes, int64_t *h_info, void *stream) {
     B3C_REQUIRE(n > 0 && nnz >= 0 && d_indptr && d_x && d_ws && h_info, "bad arguments");
     B3C_REQUIRE(nnz == 0 || (d_indices && (d_data || (d_counts && d_sites))), "null matrix arrays");
-    const bool want_packed = !d_data && d_counts && g_cnt_stream.load() == 2;
-    const KRLayout L = kr_layout(n, nnz, n, want_packed);
-    if (ws_bytes < L.total) {
-        set_error("KR workspace too small: %lld < %lld", (long long)ws_bytes, (long long)L.total);
-        return B3C_ERR_CAPACITY;
-    }
     cudaStream_t s = (cudaStream_t)stream;
     KRArgs A;
-    kr_bind(A, L, (char *)d_ws, n, 0, n, nnz, d_indptr, d_indices, d_data);
-    A.cnt32 = d_data ? nullptr : d_counts;
-    A.sites = d_data ? nullptr : d_sites;
-    A.cnt_stream = (A.cnt32 != nullptr && g_cnt_stream.load()) ? ((g_cnt_stream.load() == 2 && A.slab) ? 2 : 1) : 0;
-    KRScalars S;
-    kr_scalars_init(S, tol, delta, Delta, max_iter);
-    B3C_CUDA(cudaMemcpyAsync(A.ctl, &S, sizeof(S), cudaMemcpyHostToDevice, s));
-    B3C_CUDA(cudaMemsetAsync(A.timers, 0, sizeof(KRTimers), s));
-    int rc = kr_prepare(A, L, s);
+    KRLayout L;
+    int rc = kr_operand(A, L, n, 0, n, nnz, d_indptr, d_indices, d_data, d_counts, d_sites, tol, delta, Delta, max_iter,
+                        d_ws, ws_bytes, s);
     if (rc) return rc;
     return kr_launch_collect(A, max_iter, d_x, h_info, s);
 }
@@ -2466,20 +2521,15 @@ static int kr_run_peer_impl(int32_t n, int32_t row_lo, int32_t row_hi, int64_t n
     B3C_REQUIRE(d_indptr && d_x && d_ws && h_info && h_exchange && nnz_local >= 0, "bad arguments");
     B3C_REQUIRE(n_ranks >= 1 && n_ranks <= KR_MAX_RANKS && rank >= 0 && rank < n_ranks, "bad rank %d of %d (at most %d)",
                 rank, n_ranks, KR_MAX_RANKS);
-    const KRLayout L = kr_layout(n, nnz_local, row_hi - row_lo, !d_data && d_counts && g_cnt_stream.load() == 2);
-    if (ws_bytes < L.total) {
-        set_error("KR workspace too small: %lld < %lld", (long long)ws_bytes, (long long)L.total);
-        return B3C_ERR_CAPACITY;
-    }
+    for (int g = 0; g < n_ranks; ++g) B3C_REQUIRE(h_exchange[g] != nullptr, "null exchange buffer of rank %d", g);
     cudaStream_t s = (cudaStream_t)stream;
     KRArgs A;
-    kr_bind(A, L, (char *)d_ws, n, row_lo, row_hi, nnz_local, d_indptr, d_indices, d_data);
-    A.cnt32 = d_data ? nullptr : d_counts;
-    A.sites = d_data ? nullptr : d_sites;
-    A.cnt_stream = (A.cnt32 != nullptr && g_cnt_stream.load()) ? ((g_cnt_stream.load() == 2 && A.slab) ? 2 : 1) : 0;
+    KRLayout L;
+    int rc = kr_operand(A, L, n, row_lo, row_hi, nnz_local, d_indptr, d_indices, d_data, d_counts, d_sites, tol, delta,
+                        Delta, max_iter, d_ws, ws_bytes, s);
+    if (rc) return rc;
     const XLayout X = x_layout(n);
     for (int g = 0; g < n_ranks; ++g) {
-        B3C_REQUIRE(h_exchange[g] != nullptr, "null exchange buffer of rank %d", g);
         char *b = (char *)h_exchange[g];
         A.xflag[g] = (unsigned long long *)(b + X.o_flag);
         A.xx[g] = (double *)(b + X.o_x);
@@ -2497,12 +2547,6 @@ static int kr_run_peer_impl(int32_t n, int32_t row_lo, int32_t row_hi, int64_t n
     A.Z = A.xz[rank];
     A.part = A.xpart[rank];
     A.ll = A.xll[rank];
-    KRScalars S;
-    kr_scalars_init(S, tol, delta, Delta, max_iter);
-    B3C_CUDA(cudaMemcpyAsync(A.ctl, &S, sizeof(S), cudaMemcpyHostToDevice, s));
-    B3C_CUDA(cudaMemsetAsync(A.timers, 0, sizeof(KRTimers), s));
-    int rc = kr_prepare(A, L, s);
-    if (rc) return rc;
     return kr_launch_collect(A, max_iter, d_x, h_info, s);
 }
 
@@ -2559,6 +2603,60 @@ int b3c_spmv(int32_t n, int64_t nnz, const int64_t *d_indptr, const int32_t *d_i
     if (rc) return rc;
     k_spmv_collect<<<(unsigned)A.n_chunks, KR_THREADS, 0, s>>>(A, d_y);
     B3C_LAUNCH_CHECK();
+    return B3C_OK;
+}
+
+// ---- test hooks: the operand's layout and its row sums ------------------------------------------------
+int b3c_kr_plan(int32_t n, int64_t nnz_local, int32_t rows, int32_t counts, int64_t *h_out) {
+    B3C_REQUIRE(h_out != nullptr && n > 0 && nnz_local >= 0 && rows >= 1 && rows <= n, "bad arguments");
+    const KRLayout L = kr_layout(n, nnz_local, rows, counts && g_cnt_stream.load() == 2);
+    h_out[0] = L.slab ? L.S : 0;
+    h_out[1] = L.S;
+    h_out[2] = L.W;
+    h_out[3] = kr_cnt_stream(counts != 0, L.slab != 0);
+    h_out[4] = L.total;
+    return B3C_OK;
+}
+
+int b3c_kr_rowsum(int32_t n, int32_t row_lo, int32_t row_hi, int64_t nnz_local, const int64_t *d_indptr,
+                  const int32_t *d_indices, const double *d_data, const uint32_t *d_counts, const int32_t *d_sites,
+                  int32_t which, const double *d_v, double *d_q, void *d_ws, int64_t ws_bytes, int64_t *h_info,
+                  void *stream) {
+    B3C_REQUIRE(n > 0 && 0 <= row_lo && row_lo < row_hi && row_hi <= n, "bad row block [%d,%d) of %d", row_lo, row_hi, n);
+    B3C_REQUIRE(row_lo % CHUNK == 0 && (row_hi % CHUNK == 0 || row_hi == n), "row blocks must be %d-row aligned", CHUNK);
+    B3C_REQUIRE(d_indptr && d_v && d_q && d_ws && h_info && nnz_local >= 0 && (which == 0 || which == 1), "bad arguments");
+    B3C_REQUIRE(!d_data != !d_sites && (d_data || d_counts), "pass the values, or the counts and the sites");
+    B3C_REQUIRE(nnz_local == 0 || d_indices, "null matrix arrays");
+    cudaStream_t s = (cudaStream_t)stream;
+    KRArgs A;
+    KRLayout L;
+    int rc = kr_operand(A, L, n, row_lo, row_hi, nnz_local, d_indptr, d_indices, d_data, d_counts, d_sites, 1e-6, 0.1,
+                        3.0, 1000, d_ws, ws_bytes, s);
+    if (rc) return rc;
+    // v goes where the iteration keeps the operand it multiplies: u of a CG step (which = 0) or x of a residual
+    // (which = 1); the other pair is filled with NaN so that a row sum reading the wrong one cannot pass
+    double *opnd = which ? A.x : A.u, *scaled = which ? A.xs : A.us;
+    B3C_CUDA(cudaMemsetAsync(which ? A.u : A.x, 0xff, (size_t)L.nvec * 8, s));
+    B3C_CUDA(cudaMemsetAsync(which ? A.us : A.xs, 0xff, (size_t)L.nvec * 8, s));
+    k_kr_stage<<<(unsigned)ceil_div(n, 256), 256, 0, s>>>(n, d_v, A.inv_s, opnd, A.cnt_stream ? scaled : nullptr);
+    B3C_LAUNCH_CHECK();
+    KRArgs B = A;
+    B.u = A.cnt_stream ? scaled : opnd;
+    rc = launch_spmv(B, s);
+    if (rc) return rc;
+    k_kr_rowsum<<<(unsigned)ceil_div(row_hi - row_lo, CHUNK), KR_THREADS, 0, s>>>(A, opnd, d_q);
+    B3C_LAUNCH_CHECK();
+    KRScalars S;
+    B3C_CUDA(cudaMemcpyAsync(&S, A.ctl, sizeof(S), cudaMemcpyDeviceToHost, s));
+    B3C_CUDA(cudaStreamSynchronize(s));
+    h_info[0] = A.slab ? A.S : 0;
+    h_info[1] = A.S;
+    h_info[2] = A.cnt_stream == 2 ? 4 : A.cnt_stream ? (A.slab ? 6 : 8) : (A.slab ? 10 : 12);
+    h_info[3] = A.n_big;
+    h_info[4] = A.nnzv;
+    h_info[5] = A.n_seg;
+    h_info[6] = S.zero_diag;
+    h_info[7] = L.total;
     return B3C_OK;
 }
 

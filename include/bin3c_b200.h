@@ -179,8 +179,10 @@ int b3c_site_norm_f64(int32_t n_local, int32_t row_lo, const int64_t *d_indptr,
  * a time (see csrc/kr.cu); B3C_OPT_KR_SLAB_WIDTH caps the slab width (default 28672 columns, the most
  * that fits in a CTA's shared memory), B3C_OPT_KR_MAX_SLABS the slab count (default 16, at most 48; wider
  * matrices, or 0, select the form that gathers through L1/L2 -- except that at the default, matrices of up
- * to 48 slabs whose (row, slab) cells hold 6 or more entries on average stay in the slab form; b3c_kr_run_peer*
- * applies that rule to its own row block).  Results are
+ * to 48 slabs whose (row, slab) cells hold 6 or more entries on average -- 4 for the packed count stream -- stay in the
+ * slab form; b3c_kr_run_peer* applies that rule to its own row block, counting the block's rows rounded up to whole
+ * 1024-row chunks, as the stream lays its cells out: a tail block of fewer rows takes the form a 1024-row block with the
+ * same entries takes, which b3c_krp_workspace_bytes has room for).  Results are
  * identical up to fp64 summation order.  Workspace sizes depend on these, so set them before the *_workspace_bytes() query.
  * B3C_OPT_KR_FLAGS (default 22) is a bit set for A/B measurements: 1 = order every lane's run of the
  * stream by shared-memory bank (off: the pass costs more than it saves below ~180 SpMV per solve), 2 = align the SpMV CTA ranges with the slabs, 4 = single-word grid
@@ -213,6 +215,22 @@ int b3c_set_option(int32_t key, int64_t value);
  * keys per warp, contigs of the partial shared-memory diagonal, passes and digit bits of the key sort
  * (bits [0, 2b)), passes and digit bits of the mirror composite's sort, count bits of the composite. */
 int b3c_accum_plan(int64_t pair_capacity, int32_t n_seq, int32_t n_refs, int64_t *h_out);
+/* b3c_kr_plan: the SpMV operand layout b3c_kr_run* (rows = n) or b3c_kr_run_peer* (rows = the block's row count)
+ * chooses for a matrix of n columns and nnz_local entries under the current options (host-only, no CUDA call).
+ * counts != 0: the counts form.  h_out[5] = slabs (0 = gather form), S, slab width W, the stream form requested
+ * (0 fp64, 1 32-bit counts, 2 packed counts; the build falls back from 2 to 1 when the side list overflows), and the
+ * workspace bytes that layout needs. */
+int b3c_kr_plan(int32_t n, int64_t nnz_local, int32_t rows, int32_t counts, int64_t *h_out);
+/* b3c_kr_rowsum: builds the operand of rows [row_lo, row_hi) exactly as b3c_kr_run_peer* does ([0, n): as b3c_kr_run*)
+ * -- d_data for fp64 values, or d_counts with d_sites for the counts form (d_data null) -- and writes to d_q[row -
+ * row_lo] the row sums KR's iteration uses for the local rows, (A v)_r plus the zero-diagonal term, with v = d_v
+ * (all n columns) taken as the CG operand u (which = 0) or as x of a residual (which = 1).  Synchronises.
+ * h_info[8] = slabs (0 = gather form), S, stream bytes per entry, side-list entries, stream entries incl. padding,
+ * segments, zero diagonals of the block, workspace bytes the layout needs. */
+int b3c_kr_rowsum(int32_t n, int32_t row_lo, int32_t row_hi, int64_t nnz_local, const int64_t *d_indptr,
+                  const int32_t *d_indices, const double *d_data, const uint32_t *d_counts, const int32_t *d_sites,
+                  int32_t which, const double *d_v, double *d_q, void *d_ws, int64_t ws_bytes, int64_t *h_info,
+                  void *stream);
 
 int64_t b3c_kr_workspace_bytes(int32_t n, int64_t nnz);
 int b3c_kr_run(int32_t n, int64_t nnz, const int64_t *d_indptr, const int32_t *d_indices,

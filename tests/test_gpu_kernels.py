@@ -700,6 +700,9 @@ KR_FORMS = {
     'counts2': ('counts', 1000, 16, 2, 3),
     'counts1': ('counts', 1000, 16, 1, 3),
     'counts0': ('counts', 1000, 16, 0, 3),
+    'counts_gather': ('counts', None, 0, 2, 0),       # counts in the gather form: 32-bit counts, 8 B per entry
+    'counts_s9': ('counts', 334, 16, 2, 9),
+    'counts_s24': ('counts', 126, 48, 2, 24),         # beyond 12 slabs: the batched rounds of rows_q
 }
 
 

@@ -832,13 +832,14 @@ def test_fused_counts_form_matches_the_staged_form(dev):
         dev.check(dev.lib.b3c_set_option(5, 2))
 
 
-@pytest.mark.parametrize('offdiag_big', ['none', 'few', 'many'])
+@pytest.mark.parametrize('offdiag_big', ['none', 'few', 'many', 'cap', 'cap_plus'])
 def test_packed_count_stream_large_counts(dev, offdiag_big):
     """The packed stream (16-bit count | 16-bit column, 4 B per entry; B3C_OPT_KR_COUNT_STREAM = 2, the default in the
     slab form): diagonal counts above 65535 -- intra-contig pair counts of long contigs -- keep their low 16 bits in
     the stream and their high part as a per-row term; the high part of an OFF-diagonal count above 65535 goes to a short
     side list sorted by (row, column) that the row sums add in (rows with a zero diagonal, a large diagonal and several
-    large off-diagonal counts among them); more than 4096 such counts make the build fall back to 32-bit counts.
+    large off-diagonal counts among them); 4096 such counts (2048 upper ones mirrored, `cap`) still fit the list, and
+    more (`cap_plus`: 4098) make the build fall back to 32-bit counts.
     Either way: n_iter equal to the oracle's and to the 32-bit stream's, x <= 1e-9 (measured ~1e-15), the same bits
     when run twice, and the stream width reported."""
     import torch
@@ -860,6 +861,13 @@ def test_packed_count_stream_large_counts(dev, offdiag_big):
         diag[[40, 2000]] = 0
     elif offdiag_big == 'many':
         up = (up * 1000).tocsr()           # ~9000 of the 18000 upper entries exceed 65535
+    elif offdiag_big in ('cap', 'cap_plus'):
+        up = up.tocoo()
+        k = 2048 if offdiag_big == 'cap' else 2049
+        pick = rng.choice(up.nnz, k, replace=False)
+        data = up.data.astype(np.int64)
+        data[pick] = rng.integers(65536, 400_000, size=k)
+        up = sp.coo_matrix((data, (up.row, up.col)), shape=up.shape).tocsr()
     m = (up + up.T + sp.diags(diag, dtype=np.int64)).tocsr()
     m.eliminate_zeros()
     m = m.astype(np.uint32)
@@ -879,7 +887,7 @@ def test_packed_count_stream_large_counts(dev, offdiag_big):
         finally:
             dev.check(dev.lib.b3c_set_option(5, 2))
         got[mode] = (x.cpu().numpy().copy(), info)
-    assert got[2][1]['stream_bytes_per_entry'] == (6 if offdiag_big == 'many' else 4)
+    assert got[2][1]['stream_bytes_per_entry'] == (6 if offdiag_big in ('many', 'cap_plus') else 4)
     assert got[1][1]['stream_bytes_per_entry'] == 6
     assert got[2][1]['n_iter'] == got[1][1]['n_iter']
     assert got[2][1]['n_iter'] == it_ref
