@@ -20,6 +20,8 @@ B3C_ERR_TIE = -6
 B3C_ERR_FORMAT = -7
 
 B3C_EDGES_MAX_LINE_BYTES = 49     # the longest line b3c_edges_text writes
+B3C_BGZF_MEMBER_INPUT = 65280     # input bytes per member of b3c_bgzf_deflate
+B3C_BGZF_MEMBER_MAX = 65536       # the longest member it writes
 
 
 class B3CError(RuntimeError):
@@ -112,6 +114,9 @@ SIGNATURES = {
     'b3c_sites_finish': (C.c_int, [_p, _p, _p, _i64, _pi64, _p]),
     'b3c_edges_text_workspace_bytes': (_i64, [_i64]),
     'b3c_edges_text': (C.c_int, [_p, _i64, _p, _p, _p, _i64, _i32, _i32, _p, _i64, _pi64, _p]),
+    'b3c_bgzf_deflate_workspace_bytes': (_i64, [_i64]),
+    'b3c_bgzf_deflate': (C.c_int, [_p, _i64, _p, _i64, _p, _i64, _pi64, _p]),
+    'b3c_bgzf_inflate': (C.c_int, [_p, _i64, _p, _p, _i32, _p, _i64, _p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

@@ -5,8 +5,7 @@
 // The host reads the file in SLABS of whole BGZF blocks and lists the blocks (include/bin3c_io.h: b3c_bgzf_scan);
 // everything else happens here, one slab at a time, in a buffer U that holds the partial record the previous slab
 // ended with (the carry) followed by the inflated blocks:
-//   k_inflate  one thread per block: raw inflate (inflate.cuh), output size == ISIZE
-//   k_crc      one warp per block: CRC-32 of 32 lane pieces joined with crc32_combine, against the trailer
+//   k_inflate, k_crc   raw inflate (output size == ISIZE) and CRC-32 of every block: bgzf_inflate_blocks (bgzf.cu)
 //   k_guess    one thread per block: guess where the block's first record starts (the block start when it passes the
 //              field checks -- htslib flushes a block before a record that would not fit -- else the first offset
 //              that does) and walk the block_size chain from there to the first record start at or after the block end
@@ -22,8 +21,8 @@
 //              block its first output index, and keeps the pending first mate for the next slab
 //   k_emit     one thread per block: writes the block's records in input order
 // Errors are recorded as (stream position << 8 | code) with atomicMin, so the one reported is the first in the stream.
+#include "bgzf.cuh"
 #include "common.cuh"
-#include "inflate.cuh"
 
 namespace b3c {
 namespace {
@@ -280,58 +279,6 @@ __global__ void k_begin(Header *hd, int32_t min_mapq, int32_t strong, int32_t mi
     for (int k = 0; k < 4; ++k) hd->result[k] = 0;
     hd->in.pending = 0;
     hd->out.pending = 0;
-}
-
-__global__ void __launch_bounds__(64) k_inflate(Slab S) {
-    const int b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= S.nb) return;
-    const int64_t isize = blk_isize(S, b);
-    if (isize == 0) return;                            // the host reader does not inflate an empty block either
-    const int64_t bsize = blk_bsize(S, b);
-    const uint8_t *blk = S.comp + S.blocks[3 * b];
-    const int64_t xlen = rd16(blk + 10);
-    const int64_t plen = bsize + 1 - 12 - xlen - 8;
-    int64_t n = 0;
-    const int rc = b3c_inflate::inflate_raw(blk + 12 + xlen, plen, S.u + S.carry + S.blocks[3 * b + 2], isize, &n);
-    if (rc != b3c_inflate::OK || n != isize) record_error(S.hd, S.u0 + S.carry + S.blocks[3 * b + 2], E_INFLATE);
-}
-
-__global__ void __launch_bounds__(256) k_crc(Slab S) {
-    __shared__ uint32_t table[256];
-    for (int k = threadIdx.x; k < 256; k += blockDim.x) {
-        uint32_t c = (uint32_t)k;
-        for (int j = 0; j < 8; ++j) c = (c & 1) ? (c >> 1) ^ b3c_inflate::CRC_POLY : c >> 1;
-        table[k] = c;
-    }
-    __syncthreads();
-    const int b = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5);
-    const unsigned lane = lane_id();
-    if (b >= S.nb) return;
-    const int64_t isize = blk_isize(S, b);
-    if (isize == 0) return;
-    const uint8_t *data = S.u + S.carry + S.blocks[3 * b + 2];
-    const int64_t piece = (isize + 31) / 32;
-    const int64_t lo = min((int64_t)lane * piece, isize), hi = min(lo + piece, isize);
-    uint32_t c = ~0u;
-    for (int64_t k = lo; k < hi; ++k) c = table[(c ^ data[k]) & 0xff] ^ (c >> 8);
-    c = ~c;
-    // join the 32 pieces in order: crc(A || B) = crc(A) * x^(8 len B) + crc(B)
-    const uint32_t step = b3c_inflate::x8nmodp(piece);
-    uint32_t joined = 0;
-    for (int l = 0; l < 32; ++l) {
-        const uint32_t cl = __shfl_sync(kFullMask, c, l);
-        const int64_t llo = min((int64_t)l * piece, isize), lhi = min(llo + piece, isize);
-        if (lane == 0) {
-            if (l == 0) joined = cl;
-            else if (lhi - llo == piece) joined = b3c_inflate::multmodp(step, joined) ^ cl;
-            else joined = b3c_inflate::crc32_combine(joined, cl, lhi - llo);
-        }
-    }
-    if (lane == 0) {
-        const uint8_t *blk = S.comp + S.blocks[3 * b];
-        const uint32_t want = rd32(blk + blk_bsize(S, b) + 1 - 8);
-        if (joined != want) record_error(S.hd, S.u0 + S.carry + S.blocks[3 * b + 2], E_CRC);
-    }
 }
 
 __global__ void __launch_bounds__(128) k_guess(Slab S) {
@@ -659,11 +606,19 @@ int b3c_bamdec_slab(void *d_ws, const uint8_t *d_comp, const int64_t *d_blocks, 
     S.out = d_out;
     S.out_cap = out_capacity;
     if (n_blocks > 0) {
-        const int g64 = (int)ceil_div(n_blocks, 64), g128 = (int)ceil_div(n_blocks, 128), gw = (int)ceil_div(n_blocks, 8);
-        k_inflate<<<g64, 64, 0, s>>>(S);
-        B3C_LAUNCH_CHECK();
-        k_crc<<<gw, 256, 0, s>>>(S);
-        B3C_LAUNCH_CHECK();
+        const int g128 = (int)ceil_div(n_blocks, 128);
+        BgzfBlocks B;
+        B.comp = d_comp;
+        B.blocks = d_blocks;
+        B.nb = n_blocks;
+        B.u = d_u + carry_bytes;
+        B.u_cap = u_bytes;
+        B.err = &S.hd->err;
+        B.err_base = S.u0 + carry_bytes;
+        B.e_inflate = E_INFLATE;
+        B.e_crc = E_CRC;
+        const int rc = bgzf_inflate_blocks(B, s);
+        if (rc != B3C_OK) return rc;
         k_guess<<<g128, 128, 0, s>>>(S);
         B3C_LAUNCH_CHECK();
         k_verify<<<1, 1, 0, s>>>(S);

@@ -5,6 +5,13 @@ cPickle of the whole ContactMap after `mkmap`, bin3C.py:165; read back by `clust
     save_object(file_name, obj)                 io_utils.py:12-21   (.gz appended if missing)
     load_object(file_name)                      io_utils.py:24-32   (gzip / bz2 / plain by suffix)
     save_object(file_name, obj, stock=True)     the same file written so that a STOCK bin3C run can read it
+    save_object(file_name, obj, device=True)    the same pickle, deflated on the GPU as BGZF-framed gzip
+    load_object(file_name, device=True)         a file of save_object(device=True), inflated on the GPU
+
+The device path (include/bin3c_b200.h: b3c_bgzf_*) writes a multi-member gzip file: the pickle cut into 65280-byte
+pieces, each one gzip member with the BGZF header, then the 28-byte BGZF end-of-file member.  Python's gzip (2.7 and
+3) reads it, so load_object(device=False) and a stock `cluster` open it unchanged; the file carries no name or time
+and is the same on every run.  load_object(device=True) reads only such BGZF files.
 
 Interchange with a stock run (SURVEY section 8f-5).  A stock run is Python 2.7 + NumPy 1.14 + SciPy 1.1, and its
 classes live in `mzd.contact_map`.  A Python 3 pickle of this package's ContactMap is useless to it three times
@@ -79,8 +86,14 @@ def open_output(file_name, append=False, compress=None, gzlevel=6):
     raise RuntimeError('Unknown compression type {}'.format(compress))
 
 
-def save_object(file_name, obj, stock=False):
-    """Serialise an object to a gzip-compressed file (io_utils.py:12-21).  stock=True: readable by a stock bin3C."""
+def save_object(file_name, obj, stock=False, device=False, slab_members=None):
+    """
+    Serialise an object to a gzip-compressed file (io_utils.py:12-21).  stock=True: readable by a stock bin3C.
+    device=True: deflated on the GPU (BGZF framing, see the module docstring); slab_members = 65280-byte members per
+    host slab (default DEFAULT_SLAB_MEMBERS), which changes nothing in the file.
+    """
+    if device:
+        return _save_on_device(file_name, obj, stock, slab_members or DEFAULT_SLAB_MEMBERS)
     with open_output(file_name, compress='gzip') as out_h:
         if stock:
             out_h.write(dumps_stock(obj))
@@ -88,10 +101,179 @@ def save_object(file_name, obj, stock=False):
             pickle.dump(obj, out_h, protocol=pickle.HIGHEST_PROTOCOL)
 
 
-def load_object(file_name):
-    """Deserialise an object written by save_object here or by a stock bin3C run (io_utils.py:24-32)."""
+def load_object(file_name, device=False, slab_bytes=None):
+    """
+    Deserialise an object written by save_object here or by a stock bin3C run (io_utils.py:24-32).  device=True:
+    a file of save_object(device=True), inflated on the GPU and read slab_bytes compressed bytes at a time.
+    """
+    if device:
+        return loads(_inflate_on_device(file_name, slab_bytes or DEFAULT_LOAD_SLAB_BYTES))
     with open_input(file_name) as in_h:
         return loads(in_h.read())
+
+
+# ---- the device path: BGZF-framed gzip deflated and inflated on the GPU -------------------------------------------
+
+MEMBER_INPUT = 65280                  # pickle bytes per gzip member (include/bin3c_b200.h: B3C_BGZF_MEMBER_INPUT)
+MEMBER_MAX = 65536
+DEFAULT_SLAB_MEMBERS = 512            # 33 MB of pickle per host slab
+DEFAULT_LOAD_SLAB_BYTES = 64 << 20
+BGZF_EOF = bytes.fromhex('1f8b08040000000000ff0600424302001b0003000000000000000000')
+
+
+class _SlabWriter(object):
+    """The file object pickle writes to: fills the write-behind ring's slabs and hands each full one over."""
+
+    def __init__(self, ring, views):
+        self.ring, self.views = ring, views
+        self.k, self.n = ring.acquire(), 0
+
+    def write(self, b):
+        mv = memoryview(b).cast('B')
+        done, total = 0, len(mv)
+        while done < total:
+            a = self.views[self.k]
+            m = min(len(a) - self.n, total - done)
+            a[self.n:self.n + m] = mv[done:done + m]
+            self.n += m
+            done += m
+            if self.n == len(a):
+                self.ring.release(self.k, self.n)
+                self.k, self.n = self.ring.acquire(), 0
+        return total
+
+    def close(self):
+        if self.n:
+            self.ring.release(self.k, self.n)
+        self.n = 0
+
+
+def _cuda(what):
+    import torch
+    if not torch.cuda.is_available():
+        raise RuntimeError('{}(device=True) needs a CUDA device; the host path is device=False'.format(what))
+    return torch
+
+
+def _save_on_device(file_name, obj, stock, slab_members):
+    """
+    save_object(device=True).  pickle writes into pinned slabs of slab_members members; a write-behind slab ring
+    deflates each full slab on the device (b3c_bgzf_deflate) and writes its members to the file while the next
+    slab fills.
+    """
+    import ctypes as C
+    torch = _cuda('save_object')
+    from . import _cabi, slab_ring
+    if not file_name.endswith('.gz'):
+        file_name += '.gz'
+    k = int(slab_members)
+    assert k >= 1, 'slab_members must be positive'
+    with open(file_name, 'wb') as f:
+        dev = torch.device('cuda', torch.cuda.current_device())
+        ws = torch.empty(int(_cabi.lib.b3c_bgzf_deflate_workspace_bytes(k)), dtype=torch.uint8, device=dev)
+        d_in = torch.empty(k * MEMBER_INPUT, dtype=torch.uint8, device=dev)
+        d_out = torch.empty(k * MEMBER_MAX, dtype=torch.uint8, device=dev)
+        h_out = torch.empty(k * MEMBER_MAX, dtype=torch.uint8, pin_memory=True)
+        slabs = [torch.empty(k * MEMBER_INPUT, dtype=torch.uint8, pin_memory=True) for _ in range(2)]
+        out_bytes = C.c_int64()
+
+        def drain(slab, nbytes):                        # the ring's thread
+            with torch.cuda.device(dev):
+                stream = torch.cuda.current_stream()
+                d_in[:nbytes].copy_(slab[:nbytes], non_blocking=True)
+                _cabi.check(_cabi.lib.b3c_bgzf_deflate(ws.data_ptr(), ws.numel(), d_in.data_ptr(), nbytes,
+                                                       d_out.data_ptr(), d_out.numel(), C.byref(out_bytes),
+                                                       C.c_void_p(stream.cuda_stream)))
+                m = int(out_bytes.value)
+                h_out[:m].copy_(d_out[:m])
+            f.write(memoryview(h_out.numpy())[:m])
+
+        with slab_ring.SlabRing(slabs, drain=drain) as ring:
+            w = _SlabWriter(ring, [t.numpy() for t in slabs])
+            if stock:
+                w.write(dumps_stock(obj))
+            else:
+                pickle.dump(obj, w, protocol=pickle.HIGHEST_PROTOCOL)
+            w.close()
+        f.write(BGZF_EOF)
+
+
+def _inflate_on_device(file_name, slab_bytes):
+    """
+    The bytes of a file of save_object(device=True).  A read-ahead slab ring reads the file into two pinned slabs
+    and lists each slab's members (b3c_bgzf_scan of libbin3c_io.so) while the device inflates the previous slab
+    and checks every member's CRC-32 and ISIZE (b3c_bgzf_inflate).
+    """
+    import ctypes as C
+    torch = _cuda('load_object')
+    from . import _cabi, bam_io, slab_ring
+    cap = max(int(slab_bytes), 1) + MEMBER_MAX           # always holds one whole member
+    max_blocks = cap // 28 + 1                           # the shortest member is the end-of-file one
+    dev = torch.device('cuda', torch.cuda.current_device())
+    with open(file_name, 'rb') as f:
+        pinned = [torch.empty(cap, dtype=torch.uint8, pin_memory=True) for _ in range(2)]
+        left, eof, first = np.empty(0, dtype=np.uint8), False, [True]
+
+        def fill(a):                                     # the ring's thread: the carried bytes, then the file
+            nonlocal left, eof
+            n = len(left)
+            a[:n] = left
+            while n < cap and not eof:
+                m = f.readinto(memoryview(a)[n:cap])
+                eof = not m
+                n += m or 0
+            offs = np.empty(max_blocks, dtype=np.int64)
+            bsz = np.empty(max_blocks, dtype=np.int32)
+            isz = np.empty(max_blocks, dtype=np.int32)
+            used = np.zeros(1, dtype=np.int64)
+            nb = bam_io.lib.b3c_bgzf_scan(a.ctypes.data, n, 1 if eof else 0, offs.ctypes.data, bsz.ctypes.data,
+                                          isz.ctypes.data, max_blocks, used.ctypes.data)
+            if nb < 0:
+                msg = bam_io.last_error()
+                if first[0] and 'not a BGZF file' in msg:
+                    msg += ': load_object(device=True) reads the BGZF files of save_object(device=True); ' \
+                           'read this file with device=False'
+                raise ValueError('{}: {}'.format(file_name, msg))
+            first[0] = False
+            c = int(used[0])
+            left = a[c:n].copy()
+            last_eof = bool(nb) and isz[nb - 1] == 0 and bytes(a[offs[nb - 1]:c]) == BGZF_EOF
+            return int(nb), c, offs[:nb], bsz[:nb], isz[:nb], last_eof, eof and c == n
+
+        parts, ends_with_eof = [], False
+        stream = torch.cuda.current_stream()
+        ws = torch.empty(8, dtype=torch.uint8, device=dev)
+        d_comp = torch.empty(cap, dtype=torch.uint8, device=dev)
+        d_u = h_u = None
+        with slab_ring.SlabRing([p.numpy() for p in pinned], fill=fill) as ring:
+            for k, (nb, c, offs, bsz, isz, last_eof, last) in ring:
+                ends_with_eof = last_eof if nb else ends_with_eof
+                tbl = np.empty((nb, 3), dtype=np.int64)
+                tbl[:, 0] = offs
+                tbl[:, 1] = bsz.astype(np.int64) | (isz.astype(np.int64) << 32)
+                u_off = np.cumsum(isz, dtype=np.int64)
+                tbl[:, 2] = u_off - isz
+                u_bytes = int(u_off[-1]) if nb else 0
+                if u_bytes and (d_u is None or d_u.numel() < u_bytes):
+                    d_u = torch.empty(u_bytes, dtype=torch.uint8, device=dev)
+                    h_u = torch.empty(u_bytes, dtype=torch.uint8, pin_memory=True)
+                if c:
+                    d_comp[:c].copy_(pinned[k][:c], non_blocking=True)
+                d_tbl = torch.from_numpy(tbl.reshape(-1)).to(dev) if nb else None
+                rc = _cabi.lib.b3c_bgzf_inflate(ws.data_ptr(), ws.numel(), d_comp.data_ptr(),
+                                                d_tbl.data_ptr() if nb else None, nb,
+                                                d_u.data_ptr() if u_bytes else None, u_bytes,
+                                                C.c_void_p(stream.cuda_stream))
+                ring.release(k)                          # the call synchronised: the pinned slab is free
+                if rc == _cabi.B3C_ERR_FORMAT:
+                    raise ValueError('{}: {}'.format(file_name, _cabi.last_error()))
+                _cabi.check(rc)
+                if u_bytes:
+                    h_u[:u_bytes].copy_(d_u[:u_bytes])
+                    parts.append(h_u[:u_bytes].numpy().tobytes())
+    if not ends_with_eof:
+        raise ValueError('{}: the file does not end with the BGZF end-of-file member (truncated?)'.format(file_name))
+    return b''.join(parts)
 
 
 # ---- writer: protocol-2 opcodes for the stock stack -----------------------------------------------------------

@@ -542,6 +542,33 @@ int b3c_edges_text(void *d_ws, int64_t ws_bytes, const int32_t *d_u, const int32
                    int64_t n_edges, int32_t sep, int32_t float_style, uint8_t *d_text, int64_t text_capacity,
                    int64_t *h_bytes, void *stream);
 
+/* ------------------------------------------------------------------------------------
+ * BGZF-framed gzip of a byte stream and back (bin3c_b200/csrc/bgzf.cu, deflate.cuh): the stage hand-off
+ * file contact_map.p.gz of io_utils.save_object / load_object(device=True).  The stream is cut into
+ * MEMBERS of B3C_BGZF_MEMBER_INPUT bytes (only the last one shorter); each becomes one gzip member with
+ * the BGZF header (BC subfield holding BSIZE = member length - 1), one raw-deflate block (dynamic Huffman
+ * codes, or stored when that is not longer), CRC-32 and ISIZE.  No member exceeds B3C_BGZF_MEMBER_MAX
+ * bytes.  A member is a function of its input bytes only: the output does not depend on how a stream is
+ * split into calls, as long as each call but the last passes a multiple of B3C_BGZF_MEMBER_INPUT bytes.
+ * Any gzip reader reads the members; the 28-byte BGZF end-of-file member is the caller's to append.
+ *
+ *   deflate_workspace_bytes  scratch for calls of up to max_members members
+ *   deflate    d_in[0 .. n_bytes) (device) -> whole members at d_out[0 .. *h_out_bytes) (device, any
+ *              alignment), out_capacity >= B3C_BGZF_MEMBER_MAX * members.  Synchronises the stream once.
+ *   inflate    d_comp = whole members (device), d_blocks = int64[3 n_blocks] as b3c_bamdec_slab takes
+ *              it (offset in d_comp, BSIZE | ISIZE << 32, offset of the member's inflated bytes in d_out;
+ *              b3c_bgzf_scan of include/bin3c_io.h lists them).  Each member is inflated and its ISIZE
+ *              and CRC-32 checked; a mismatch -> B3C_ERR_FORMAT, b3c_last_error() naming the first bad
+ *              member's uncompressed offset.  d_ws: 8 bytes of device scratch.  Synchronises once.
+ * ------------------------------------------------------------------------------------ */
+#define B3C_BGZF_MEMBER_INPUT 65280
+#define B3C_BGZF_MEMBER_MAX 65536
+int64_t b3c_bgzf_deflate_workspace_bytes(int64_t max_members);
+int b3c_bgzf_deflate(void *d_ws, int64_t ws_bytes, const uint8_t *d_in, int64_t n_bytes, uint8_t *d_out,
+                     int64_t out_capacity, int64_t *h_out_bytes, void *stream);
+int b3c_bgzf_inflate(void *d_ws, int64_t ws_bytes, const uint8_t *d_comp, const int64_t *d_blocks,
+                     int32_t n_blocks, uint8_t *d_out, int64_t out_capacity, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
