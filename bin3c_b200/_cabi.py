@@ -134,20 +134,24 @@ def last_error():
     return lib.b3c_last_error().decode('utf-8', 'replace')
 
 
+def error(rc, msg):
+    """The exception for a nonzero b3c_status: the type the reference raises for the same condition."""
+    if rc == B3C_ERR_ARG:
+        return AssertionError(msg)                  # the reference asserts on bad arguments
+    if rc == B3C_ERR_TIE:
+        return ValueError(msg)                      # np.amin of an empty selection (Q13)
+    if rc == B3C_ERR_FORMAT:
+        return ValueError(msg)                      # malformed BAM file: what the host reader raises for it
+    if rc in (B3C_ERR_NOCONV, B3C_ERR_NAN):
+        return RuntimeError(msg)                    # sparse_utils.py:193,214
+    return B3CError('b3c status {}: {}'.format(rc, msg))
+
+
 def check(rc):
-    """Map a b3c_status to the exception type the reference raises for the same condition."""
+    """Raise error(rc, last_error()) unless rc is B3C_OK."""
     if rc == B3C_OK:
         return
-    msg = last_error()
-    if rc == B3C_ERR_ARG:
-        raise AssertionError(msg)                   # the reference asserts on bad arguments
-    if rc == B3C_ERR_TIE:
-        raise ValueError(msg)                       # np.amin of an empty selection (Q13)
-    if rc == B3C_ERR_FORMAT:
-        raise ValueError(msg)                       # malformed BAM file: what the host reader raises for it
-    if rc in (B3C_ERR_NOCONV, B3C_ERR_NAN):
-        raise RuntimeError(msg)                     # sparse_utils.py:193,214
-    raise B3CError('b3c status {}: {}'.format(rc, msg))
+    raise error(rc, last_error())
 
 
 def launch_count():

@@ -546,6 +546,24 @@ class _Trace(object):
             self.t = now
 
 
+def _raise_kr_status(status, n_iter, max_iter):
+    """Raise what b3c_kr_run* raises for the same outcome of the iteration: the exception type _cabi.check gives the
+    status, with the message kr.cu's set_error writes for it (b3c_krp_state reports the status without a message)."""
+    if status == 0 and n_iter <= max_iter:
+        return
+    from . import _cabi
+    if status == _cabi.B3C_ERR_TIE:
+        msg = 'KR: max(ynew) == Delta with no element above Delta (reference raises ValueError here)'
+    elif status == _cabi.B3C_ERR_NAN:
+        msg = 'scale vector has developed invalid values (NANs)!'
+    elif status in (0, _cabi.B3C_ERR_NOCONV):
+        status = _cabi.B3C_ERR_NOCONV
+        msg = 'matrix balancing failed to converge in {} iterations'.format(n_iter)
+    else:
+        msg = 'KR phase loop ended with status {}'.format(status)
+    raise _cabi.error(status, msg)
+
+
 class ShardedHotPath(object):
     """The whole path over `comm.world` ranks.  Each rank passes its own chunk of pair records."""
 
@@ -676,10 +694,7 @@ class ShardedHotPath(object):
             z = torch.tensor([st['zero_diag']], dtype=torch.int64, device=eng.x.device)
             st['zero_diag'] = int(comm.all_reduce(z, 'sum').cpu()[0])
         self.kr_info = st
-        if st['status'] == -6:
-            raise ValueError('KR: max(ynew) == Delta with no element above Delta (Q13)')
-        if st['status'] != 0 or st['n_iter'] > self.kr_params[3]:
-            raise RuntimeError('matrix balancing failed to converge in {} iterations'.format(st['n_iter']))
+        _raise_kr_status(st['status'], st['n_iter'], self.kr_params[3])
         # x: every rank wrote its own slice; assemble the whole vector
         xs = eng.x
         if peer:
